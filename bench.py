@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: VQA pairs/sec of the fused eval-mode VQAModel.forward on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 256] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 256] [--impl reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK/LOCAL_RANK/WORLD_SIZE).  Workload = BASELINE.json
 configs[1]: batch 256 per GPU, 224x224 images, 20-token questions, 1000 answers, bf16 engine,
@@ -15,6 +15,10 @@ region).  ``--impl reference`` times the reference's own CPU implementation on t
 same metric: the UNMODIFIED reference when it is staged (oracle/_ref/reference.zip, written by
 tools/stage_reference.sh in the build container; ``kind: "reference"``), else the oracle port
 (``kind: "port"``).
+
+``--dump-outputs DIR`` writes the logits of the last timed step of ``value`` as DIR/logits.npy; inputs and weights
+are seeded, so two builds of the project can be compared output for output.  With several GPUs the file holds rank
+0's shard of the batch.
 """
 from __future__ import annotations
 
@@ -45,6 +49,21 @@ def measured_peaks():
         return {"hbm_gbs": d["hbm_gbs"], "bf16_tflops": d["bf16_tflops"],
                 "bf16_tflops_sustained": d.get("bf16_tflops_sustained", d["bf16_tflops"]), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
+
+
+DUMP_MAX_BYTES = 60 * 10**6     # below 64 MB with room for the .npy header
+
+
+def dump_logits(out_dir: str, logits) -> None:
+    """Write fp32 ``logits`` [B, N] as ``out_dir/logits.npy``.  A batch too large for DUMP_MAX_BYTES keeps a fixed,
+    seeded sample of its rows (sorted), the same rows on every run with the same arguments."""
+    import numpy as np
+    a = logits.float().cpu().numpy()
+    cap = DUMP_MAX_BYTES // a[0].nbytes
+    if a.shape[0] > cap:
+        a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], cap, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), a)
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -214,12 +233,12 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(args.steps, 1), max(args.warmup, 1)
-    r = cpu_reference_run(min(steps, 8), min(warmup, 2))
-    sample = (f"{min(steps, 8)} timed fp32 forwards of batch {r['batch']} (BASELINE configs[0]) on the host CPU, "
+    steps, warmup = args.steps, max(args.warmup, 1)
+    r = cpu_reference_run(steps, min(warmup, 2))
+    sample = (f"{steps} timed fp32 forwards of batch {r['batch']} (BASELINE configs[0]) on the host CPU, "
               + ("the unmodified reference VQAModel" if r["kind"] == "reference" else "oracle port of the reference forward"))
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "pairs/s", "n_gpus": args.gpus,
-            "steps": min(steps, 8), "warmup": min(warmup, 2), "ms_per_step": r["ms_per_step"],
+            "steps": steps, "warmup": min(warmup, 2), "ms_per_step": r["ms_per_step"],
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": WORKLOAD, "batch_per_step": r["batch"], "device": "host CPU"},
             "cpu_baseline": {"value": r["value"], "unit": "pairs/s", "cores": r["cores"], "kind": r["kind"],
@@ -343,6 +362,8 @@ def run_b200(args):
             barrier()
         launches = launches_per_step * K
         ms = reduce_max(e0.elapsed_time(e1))
+        if args.dump_outputs and rank == 0:     # step K-1 ran on lane (K-1) % LANES, into that lane's own buffer
+            dump_logits(args.dump_outputs, lane_out[(K - 1) % LANES])
     clocks.stop()
     if args.quick:    # A/B experiments: device-resident throughput only (not a bench line)
         if rank == 0:
@@ -851,7 +872,13 @@ def main():
     ap.add_argument("--dump-ops", default="")
     ap.add_argument("--agreement", type=int, default=0)
     ap.add_argument("--quick", action="store_true", help="device-resident throughput only (A/B experiments)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the logits of the last timed step as DIR/logits.npy (rank 0's shard with several GPUs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.agreement):
+        ap.error("--dump-outputs writes the B200 timed path's logits; --impl reference and --agreement do not run it")
     if args.impl == "reference":
         return run_reference(args)
     if args.agreement:

@@ -7,8 +7,9 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
 
+from oracle.ref_loader import reference_path  # noqa: E402
+
 GOLDEN = os.path.join(REPO, "tests", "golden")
-REFERENCE = os.environ.get("VQA_REFERENCE", "/root/reference")
 
 
 def pytest_configure(config):
@@ -22,17 +23,22 @@ def golden_meta():
         return json.load(f)
 
 
+NO_REFERENCE = "needs the original project's sources: $VQA_REFERENCE or oracle/_ref/reference.zip"
+
+
 def have_reference():
-    return os.path.isdir(os.path.join(REFERENCE, "models"))
+    return reference_path() is not None
 
 
 @pytest.fixture(scope="session")
 def reference_modules(tmp_path_factory):
-    """Import the live reference (build container only); skipped where it is absent."""
-    if not have_reference():
-        pytest.skip("reference sources not present on this machine")
+    """Import the original project from where oracle/ref_loader.py finds it (a source directory or the archive
+    tools/stage_reference.sh stages); skipped where neither is present."""
+    path = reference_path()
+    if path is None:
+        pytest.skip(NO_REFERENCE)
     os.chdir(tmp_path_factory.mktemp("refcwd"))  # utils.config mkdirs relative to CWD (SURVEY T9)
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
+    if path not in sys.path:
+        sys.path.insert(0, path)
     import importlib
     return importlib

@@ -6,7 +6,7 @@ import time
 import pytest
 import torch
 
-from conftest import REPO, have_reference
+from conftest import NO_REFERENCE, REPO, have_reference
 
 sys.path.insert(0, REPO)
 from vqa_b200.batcher import MicroBatcher  # noqa: E402
@@ -104,7 +104,7 @@ def test_confusion_matrix_and_per_class_accuracy():
     assert M.get_per_class_accuracy(conf).tolist() == [0.5, 1.0, pytest.approx(2 / 3), 0.0]
 
 
-@pytest.mark.skipif(not have_reference(), reason="reference sources not present on this machine")
+@pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 def test_metric_helpers_match_the_reference(reference_modules):
     ref = reference_modules.import_module("utils.metrics")
     g = torch.Generator().manual_seed(3)

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, REPO, have_reference
+from conftest import GOLDEN, NO_REFERENCE, REPO, have_reference
 
 sys.path.insert(0, REPO)
 from oracle import vqa_oracle as O  # noqa: E402
@@ -94,7 +94,7 @@ def test_mask_dtype_and_padding_invariance(golden_meta):
     assert torch.equal(a, c)
 
 
-@pytest.mark.skipif(not have_reference(), reason="live reference only in the build container")
+@pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 def test_oracle_matches_live_reference(reference_modules):
     ref = reference_modules.import_module("models.vqa_model")
     torch.manual_seed(11)
@@ -118,7 +118,7 @@ def test_oracle_matches_live_reference(reference_modules):
     torch.testing.assert_close(got2, want2, rtol=1e-4, atol=2e-5)
 
 
-@pytest.mark.skipif(not have_reference(), reason="live reference only in the build container")
+@pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 def test_seeded_construction_is_bit_identical_to_reference(reference_modules):
     ref = reference_modules.import_module("models.vqa_model")
     for kw in ({}, dict(use_se_attention=False, use_spatial_attention=False, use_gating=False,

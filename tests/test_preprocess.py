@@ -32,8 +32,8 @@ def test_resize_is_bit_exact_with_reference(g, name):
     """uint8 result of the PIL antialiased bilinear resize is bit-exact; the float output's moments match."""
     inf = VQAInference()
     img = Image.fromarray(g[f"{name}.u8"], "RGB")
-    u8 = inf.preprocess_image_u8(img)
-    assert np.array_equal(u8.numpy(), g[f"{name}.resized_u8"])
+    u8 = inf.preprocess_image_u8(img)          # a CUDA tensor where a GPU resizes it, else PIL's result on the host
+    assert np.array_equal(u8.cpu().numpy(), g[f"{name}.resized_u8"])
     t64 = inf.preprocess_image(img).double()
     np.testing.assert_allclose([float(t64.sum()), float(t64.abs().sum())], g[f"{name}.out_moments"], rtol=1e-6)
 

@@ -9,7 +9,7 @@ from hypothesis import given, settings, strategies as st
 
 from vqa_b200.text import AnswerVocabulary, Tokenizer
 
-from conftest import have_reference
+from conftest import NO_REFERENCE, have_reference
 
 
 @pytest.fixture(scope="module")
@@ -100,7 +100,7 @@ def test_answer_vocab(tu, tmp_path):
 _text = st.text(alphabet=st.sampled_from(list("abcXYZ 019_'?!,.\t\n-éß中")), max_size=80)
 
 
-@pytest.mark.skipif(not have_reference(), reason="live reference only in the build container")
+@pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 @settings(max_examples=300, deadline=None)
 @given(text=_text, special=st.booleans(), pad=st.booleans(), trunc=st.booleans())
 def test_property_encode_matches_live_reference(reference_modules, text, special, pad, trunc):
@@ -118,7 +118,7 @@ def test_property_encode_matches_live_reference(reference_modules, text, special
     assert a.decode(ra[0]) == b.decode(rb[0])
 
 
-@pytest.mark.skipif(not have_reference(), reason="live reference only in the build container")
+@pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 @settings(max_examples=200, deadline=None)
 @given(ans=_text)
 def test_property_answer_preprocess_matches_live_reference(reference_modules, ans):

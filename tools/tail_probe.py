@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0,'/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from vqa_b200.model import VQAModel
 from vqa_b200.synth import synth_batch
 torch.manual_seed(0)
