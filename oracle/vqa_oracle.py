@@ -70,11 +70,16 @@ def stem(sd, x, p="image_encoder.stem"):
     return F.max_pool2d(x, kernel_size=3, stride=2, padding=1)
 
 
-def residual_block(sd, p, x, stride):
-    """ResidualBlock.forward (models/cnn_backbone.py:164-197)."""
+def block_conv1(sd, p, x, stride):
+    """First half of ResidualBlock.forward (models/cnn_backbone.py:164-197): conv1 -> bn1 -> ReLU."""
     out = F.conv2d(x, sd[p + ".conv1.weight"], None, stride=stride, padding=1)
-    out = F.relu(_bn(sd, p + ".bn1", out))
-    out = F.conv2d(out, sd[p + ".conv2.weight"], None, stride=1, padding=1)
+    return F.relu(_bn(sd, p + ".bn1", out))
+
+
+def block_tail(sd, p, x, mid, stride):
+    """Second half of ResidualBlock.forward (models/cnn_backbone.py:164-197): conv2 -> bn2 on ``mid`` (the output of
+    block_conv1), plus the identity or downsampled shortcut of the block input ``x``, then ReLU."""
+    out = F.conv2d(mid, sd[p + ".conv2.weight"], None, stride=1, padding=1)
     out = _bn(sd, p + ".bn2", out)
     if (p + ".downsample.0.weight") in sd:  # built at models/cnn_backbone.py:243-249
         idn = F.conv2d(x, sd[p + ".downsample.0.weight"], None, stride=stride)
@@ -84,21 +89,35 @@ def residual_block(sd, p, x, stride):
     return F.relu(out + idn)
 
 
-def se_attention(sd, p, x):
-    """SEAttention.forward (models/attention_modules.py:91-136); no biases (:84-85)."""
+def residual_block(sd, p, x, stride):
+    """ResidualBlock.forward (models/cnn_backbone.py:164-197)."""
+    return block_tail(sd, p, x, block_conv1(sd, p, x, stride), stride)
+
+
+def se_scale(sd, p, x):
+    """The per-channel scale [B, C] of SEAttention.forward (models/attention_modules.py:91-136); no biases (:84-85)."""
     sq = x.mean(dim=(2, 3))
     ex = F.relu(F.linear(sq, sd[p + ".fc1.weight"]))
-    sc = torch.sigmoid(F.linear(ex, sd[p + ".fc2.weight"]))
-    return x * sc.view(x.shape[0], -1, 1, 1)
+    return torch.sigmoid(F.linear(ex, sd[p + ".fc2.weight"]))
 
 
-def spatial_attention(sd, p, x):
-    """SpatialAttention.forward (models/attention_modules.py:198-243); [max, avg] order (:230)."""
+def se_attention(sd, p, x):
+    """SEAttention.forward (models/attention_modules.py:91-136)."""
+    return x * se_scale(sd, p, x).view(x.shape[0], -1, 1, 1)
+
+
+def spatial_map(sd, p, x):
+    """The sigmoid attention map [B, 1, H, W] of SpatialAttention.forward (models/attention_modules.py:198-243);
+    [max, avg] order (:230)."""
     mx = x.max(dim=1, keepdim=True)[0]
     av = x.mean(dim=1, keepdim=True)
     w = sd[p + ".conv.weight"]
-    amap = torch.sigmoid(F.conv2d(torch.cat([mx, av], dim=1), w, None, padding=w.shape[-1] // 2))
-    return x * amap
+    return torch.sigmoid(F.conv2d(torch.cat([mx, av], dim=1), w, None, padding=w.shape[-1] // 2))
+
+
+def spatial_attention(sd, p, x):
+    """SpatialAttention.forward (models/attention_modules.py:198-243)."""
+    return x * spatial_map(sd, p, x)
 
 
 def residual_stage(sd, p, x, stride, taps=None):
@@ -160,23 +179,32 @@ def _mha(q, k, v, num_heads, key_mask=None):
     return ctx, w
 
 
-def text_encoder(sd, token_ids, attention_mask, num_heads, p="text_encoder"):
-    """TransformerTextEncoder.forward (models/text_encoder.py:479-529)."""
+def text_embed(sd, token_ids, p="text_encoder"):
+    """Token embedding * sqrt(D) + sinusoidal position (models/text_encoder.py:504-507, :108-112)."""
     emb = sd[p + ".token_embedding.weight"]
     D = emb.shape[1]
     x = F.embedding(token_ids, emb) * math.sqrt(D)                      # :504-507
-    x = x + sd[p + ".positional_encoding.pe"][:, : x.shape[1], :]        # :108-112
+    return x + sd[p + ".positional_encoding.pe"][:, : x.shape[1], :]     # :108-112
+
+
+def text_layer(sd, lp, x, attention_mask, num_heads):
+    """One pre-norm encoder layer of TransformerTextEncoder (models/text_encoder.py:390-397)."""
+    n = _ln(sd, lp + ".norm1", x)                                        # pre-norm, :390
+    q = _lin(sd, lp + ".self_attention.W_q", n)
+    k = _lin(sd, lp + ".self_attention.W_k", n)
+    v = _lin(sd, lp + ".self_attention.W_v", n)
+    ctx, _ = _mha(q, k, v, num_heads, attention_mask)
+    x = x + _lin(sd, lp + ".self_attention.W_o", ctx)                    # :392
+    n = _ln(sd, lp + ".norm2", x)                                        # :395
+    return x + _lin(sd, lp + ".ffn.fc2", F.relu(_lin(sd, lp + ".ffn.fc1", n)))  # :320-323,:397
+
+
+def text_encoder(sd, token_ids, attention_mask, num_heads, p="text_encoder"):
+    """TransformerTextEncoder.forward (models/text_encoder.py:479-529)."""
+    x = text_embed(sd, token_ids, p)
     layer = 0
     while (p + f".layers.{layer}.norm1.weight") in sd:
-        lp = p + f".layers.{layer}"
-        n = _ln(sd, lp + ".norm1", x)                                    # pre-norm, :390
-        q = _lin(sd, lp + ".self_attention.W_q", n)
-        k = _lin(sd, lp + ".self_attention.W_k", n)
-        v = _lin(sd, lp + ".self_attention.W_v", n)
-        ctx, _ = _mha(q, k, v, num_heads, attention_mask)
-        x = x + _lin(sd, lp + ".self_attention.W_o", ctx)                # :392
-        n = _ln(sd, lp + ".norm2", x)                                    # :395
-        x = x + _lin(sd, lp + ".ffn.fc2", F.relu(_lin(sd, lp + ".ffn.fc1", n)))  # :320-323,:397
+        x = text_layer(sd, p + f".layers.{layer}", x, attention_mask, num_heads)
         layer += 1
     enc = _ln(sd, p + ".final_norm", x)                                  # :519
     if attention_mask is not None:                                       # :523-527
@@ -220,6 +248,15 @@ def fusion(sd, feats, text_features, text_mask, num_heads, p="fusion"):
         q, w = cross_layer(sd, p + f".cross_attention.layers.{layer}", q, img, num_heads)
         weights.append(w)
         layer += 1
+    fused, att_pooled, txt_pooled = fusion_tail(sd, q, text_features, text_mask, p)
+    aux = {"cross_attention_weights": weights, "image_projected": img,
+           "attended_pooled": att_pooled, "text_pooled": txt_pooled}
+    return fused, aux
+
+
+def fusion_tail(sd, q, text_features, text_mask, p="fusion"):
+    """MultimodalFusion.forward after the cross-attention layers (models/fusion.py:303-326): masked mean pools of the
+    attended and the plain text features, gate (or sum), output LayerNorm -> (fused, att_pooled, txt_pooled)."""
     if text_mask is not None:                                            # :303-313
         m = text_mask.unsqueeze(-1).float()
         den = m.sum(dim=1).clamp(min=1)
@@ -233,10 +270,7 @@ def fusion(sd, feats, text_features, text_mask, num_heads, p="fusion"):
         fused = g * att_pooled + (1 - g) * txt_pooled
     else:
         fused = att_pooled + txt_pooled                                  # :322
-    fused = _ln(sd, p + ".output_norm", fused)                           # :326
-    aux = {"cross_attention_weights": weights, "image_projected": img,
-           "attended_pooled": att_pooled, "text_pooled": txt_pooled}
-    return fused, aux
+    return _ln(sd, p + ".output_norm", fused), att_pooled, txt_pooled   # :326
 
 
 def answer_head(sd, fused, p="answer_head.classifier"):

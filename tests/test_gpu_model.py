@@ -9,6 +9,7 @@ import torch
 pytestmark = pytest.mark.gpu
 
 from conftest import GOLDEN, REPO  # noqa: E402
+import layer_parity as LP  # noqa: E402
 
 sys.path.insert(0, REPO)
 from oracle import vqa_oracle as O  # noqa: E402
@@ -61,28 +62,6 @@ def test_forward_matches_reference_golden(golden_meta, case):
     np.testing.assert_allclose(top_p.cpu().numpy(), g["top_probs"], rtol=2e-2, atol=1e-4)
 
 
-def _grid_nchw(prog, name, H, W, C):
-    """A padded-flat NHWC workspace buffer (program.py, "HBM layout") as an NCHW fp32 tensor of the valid pixels."""
-    t = prog.tensor(name).float().cpu()
-    B = t.shape[0] // ((H + 1) * (W + 1))
-    return t.view(B, H + 1, W + 1, C)[:, :H, :W, :].permute(0, 3, 1, 2).contiguous()
-
-
-def _phases_nchw(prog, name, H, W, C):
-    """The 4-phase split a stage tail writes for the next stage's stride-2 convolution (phase (ph,pw) holds
-    x[2a+ph, 2b+pw] on the half-resolution padded grid) back to NCHW [B, C, H, W]."""
-    t = prog.tensor(name).float().cpu()
-    h2, w2 = H // 2, W // 2
-    rows = t.shape[0] // 4
-    B = rows // ((h2 + 1) * (w2 + 1))
-    out = torch.zeros(B, C, H, W)
-    for ph in range(2):
-        for pw in range(2):
-            q = t[(ph * 2 + pw) * rows: (ph * 2 + pw + 1) * rows].view(B, h2 + 1, w2 + 1, C)[:, :h2, :w2, :]
-            out[:, :, ph::2, pw::2] = q.permute(0, 3, 1, 2)
-    return out
-
-
 @pytest.mark.parametrize("case", ["default_b4", "plain_b2", "ablate_b3", "nospatial_b2"])
 def test_backbone_stage_taps_match_golden(golden_meta, case):
     """VERDICT r1: logits barely see the image (SURVEY T11), so a backbone bug could hide behind the logit gate.  The
@@ -95,15 +74,16 @@ def test_backbone_stage_taps_match_golden(golden_meta, case):
     with torch.no_grad():
         _, _, _, prog = model.engine().run(img.cuda(), ids.cuda(), mask.cuda())
     torch.cuda.synchronize()
-    got = {"stem": _grid_nchw(prog, "s1.in", 56, 56, 64)}
-    for s, (hw, c) in enumerate(((56, 64), (28, 128), (14, 256), (7, 512)), start=1):
-        got[f"stage{s}.blocks"] = _grid_nchw(prog, f"s{s}.b1.out", hw, hw, c)
+    got = {"stem": LP.grid_nchw(prog, "s1.in", 56, 56)[0]}
+    for s, hw in enumerate((56, 28, 14, 7), start=1):
+        got[f"stage{s}.blocks"] = LP.grid_nchw(prog, f"s{s}.b1.out", hw, hw)[0]
         if s < 4:
-            got[f"stage{s}"] = _phases_nchw(prog, f"s{s + 1}.in", hw, hw, c)
+            got[f"stage{s}"] = LP.phases_nchw(prog, f"s{s + 1}.in", hw, hw)[0]
         else:
-            got[f"stage{s}"] = _grid_nchw(prog, prog.feat_name, hw, hw, c)
+            got[f"stage{s}"] = LP.grid_nchw(prog, prog.feat_name, hw, hw)[0]
     errs = {}
     for k, v in got.items():
+        v = v.float().cpu()
         want = torch.from_numpy(g[f"tap.{k}.sample"])
         sample = v.flatten()[::997]
         assert sample.shape == want.shape, (k, sample.shape, want.shape)
