@@ -238,3 +238,79 @@ def test_accuracy_counters_match_reference_golden():
         idx.update(logits.argmax(-1).cuda(), targets.cuda())
         r1 = idx.compute()
         assert [r1["correct"], round(r1["accuracy_top5"] * r1["total"]), r1["total"]] == g["index_form"]
+
+
+def _special_rows(N):
+    """(logits [R, N], targets [R]): rows with NaN, +-inf and signed zeros, each with the targets that probe them."""
+    nan, inf = float("nan"), float("inf")
+    base = torch.randn(N, generator=torch.Generator().manual_seed(N))
+    rows, targets = [], []
+
+    def add(row, *ts):
+        for t in ts:
+            rows.append(row)
+            targets.append(t)
+
+    add(torch.full((N,), nan), 0, 1, 3, N - 1)                        # all NaN: only index 0 is the argmax
+    r = base.clone()
+    r[5] = nan
+    add(r, 5, 2)                                                      # a NaN target: rank 0
+    r = base.clone()
+    r[[N - 3, 9]] = nan
+    add(r, N - 3, 9, int(base.argmax()))                              # two NaNs; the finite maximum ranks third
+    r = torch.zeros(N)
+    r[[0, 2, 3]] = torch.tensor([0.1, 0.3, 0.2])
+    r[[1, 4]] = nan
+    add(r, 1, 2, 4)                                                   # pred is the first NaN, not the largest finite value
+    r = base.clone()
+    r[[4, 11]] = inf
+    r[[2, 6]] = -inf
+    add(r, 11, 4, 6, 2)                                               # +inf ties go to the lower index; -inf ranks last
+    r = torch.full((N,), -1.0)
+    r[8], r[3] = -0.0, 0.0
+    add(r, 8, 3)                                                      # -0.0 ties +0.0
+    add(torch.full((N,), -inf), 0, N - 1)
+    add(base, -1, N)                                                  # unknown answers: never correct, still counted
+    return torch.stack(rows), torch.tensor(targets)
+
+
+@pytest.mark.parametrize("N", [37, 40, 1000])
+def test_accuracy_kernel_follows_argmax_on_nan_and_inf_rows(N):
+    """Rank order NaN > +inf > finite > -inf, equal keys to the lower index: pred_out is torch.argmax (the first NaN of a
+    row that has one), rank_out is the exact rank, and top-1 / top-k hits follow from the rank.  N = 37 reads the row
+    with scalar loads, N = 40 and 1000 with 16-byte loads."""
+    from topk_ref import ref_rank
+    logits, targets = _special_rows(N)
+    B = logits.shape[0]
+    for k in (1, 2, 5):
+        c = torch.zeros(3, dtype=torch.int64, device="cuda")
+        pred = torch.full((B,), -7, dtype=torch.int64, device="cuda")
+        rank = torch.full((B,), -7, dtype=torch.int32, device="cuda")
+        accuracy_update(logits.cuda(), targets.cuda(), c, k=k, pred_out=pred, rank_out=rank)
+        want_rank = ref_rank(logits, targets)
+        assert torch.equal(pred.cpu(), torch.argmax(logits, dim=1))
+        assert torch.equal(rank.cpu().long(), want_rank)
+        valid = (targets >= 0) & (targets < N)
+        assert c.tolist() == [int((valid & (want_rank == 0)).sum()), int((valid & (want_rank < k)).sum()), B]
+        assert c.tolist()[0] == int((torch.argmax(logits, dim=1) == targets).sum())
+
+
+def test_evaluate_with_a_fully_masked_question(model):
+    """A question whose mask is all zero has a NaN logit row (as in the reference); evaluate() must count it the way
+    torch.argmax does and never report a predicted index outside the answer range."""
+    batches = []
+    for i in range(2):
+        u8, img, ids, mask = synth_batch(4, 900 + i)
+        batches.append({"images": img, "token_ids": ids, "attention_mask": mask})
+    batches[1]["attention_mask"][2] = 0
+    with torch.no_grad():
+        logits = torch.cat([model(b["images"].cuda(), b["token_ids"].cuda(), b["attention_mask"].cuda())[0].cpu()
+                            for b in batches])
+    assert bool(torch.isnan(logits[6]).all()) and int(torch.isnan(logits).any(1).sum()) == 1
+    answers = logits.nan_to_num(nan=-1.0).argmax(-1)                  # right for every finite row
+    answers[6] = 3                                                    # wrong for the NaN row (argmax 0)
+    for i, b in enumerate(batches):
+        b["answers"] = answers[4 * i: 4 * i + 4]
+    res = evaluate(model, batches)
+    assert res["total_samples"] == 8 and res["correct"] == int((logits.argmax(-1) == answers).sum()) == 7
+    assert res["common_errors"] == [{"predicted_idx": 0, "target_idx": 3, "count": 1}]

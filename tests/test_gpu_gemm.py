@@ -381,14 +381,17 @@ def test_mlp_chain(T, F, Nn, max_ctas, cs):
         G.report(f"chain y T{T} Nn{Nn}", G.named(gpu, "y"), G.named(cpu, "y"), atol=6e-3, rtol=4e-3)
 
 
-@pytest.mark.parametrize("M,N,k", [(256, 1000, 5), (1, 1000, 5), (300, 1000, 8), (130, 136, 1), (1024, 1000, 5), (64, 3128, 3)])
+@pytest.mark.parametrize("M,N,k", [(256, 1000, 5), (1, 1000, 5), (300, 1000, 8), (130, 136, 1), (1024, 1000, 5), (64, 3128, 3),
+                                   (5, 4, 4), (3, 8, 8)])
 def test_linear_with_fused_softmax_topk(M, N, k):
     """The answer head's last Linear with softmax + top-k in its epilogue (models/vqa_model.py:336-337,
-    api/inference.py:231-234) against softmax().topk() of the SAME logits: winners bit-exact (ties go to the lower index,
-    NaN ranks first like torch.topk), probabilities to fp32 rounding; rows with -inf, duplicated maxima and NaN; the
-    launch is repeated so the arrival counters must have been reset by the merging CTA."""
+    api/inference.py:231-234) against the stable rank order (tests/topk_ref.py: NaN > +inf > finite > -inf, ties to the
+    lower index) and the fp64 softmax of the SAME logits; rows with -inf, duplicated maxima, all NaN, one NaN and +inf;
+    k = N; the launch is repeated so the arrival counters must have been reset by the merging CTA."""
     import gpu_util as G
+    from topk_ref import ref_order, ref_softmax
     K = 256
+    special = M > 4 and N > 40
 
     def build(device):
         gen = torch.Generator().manual_seed(11)
@@ -399,12 +402,17 @@ def test_linear_with_fused_softmax_topk(M, N, k):
         if N > 40:
             w[7] = w[3]                       # two identical logit columns: a tie in every row
             w[N - 1] = w[N - 2]
-        W.add("w.h", w, torch.float16)
         bias = torch.zeros(npad)
         bias[:N] = torch.randn(N, generator=gen)
         if N > 40:
             bias[7], bias[N - 1] = bias[3], bias[N - 2]
             bias[11] = float("-inf")          # a column nobody may pick before the finite ones
+        if special:
+            # +inf weights in columns 13 and 17 meet inputs of one sign per row: -inf there in every row, except
+            # row 3, where +inf meets column 13's -inf bias (one NaN), and row 4, which gets +inf in column 17
+            w[13, 5] = w[17, 9] = float("inf")
+            bias[13] = float("-inf")
+        W.add("w.h", w, torch.float16)
         W.add("b", bias, torch.float32)
         W.finalize()
         ol = P.OpList(W, device)
@@ -414,6 +422,9 @@ def test_linear_with_fused_softmax_topk(M, N, k):
                   topk=(k, P.ExtRef(P.EXT["top_idx"]), P.ExtRef(P.EXT["top_probs"])))
         ol.commit()
         av = torch.randn(M, K, generator=gen)
+        if special:
+            av[:, [5, 9]] = -(av[:, [5, 9]].abs() + 0.1)
+            av[3, 5], av[4, 9] = 1.0, 1.0
         if M > 2:
             av[2] = float("nan")              # an all-NaN row (a fully masked question in the reference)
         G.named(ol, "a").copy_(av.to(torch.float16))
@@ -424,19 +435,25 @@ def test_linear_with_fused_softmax_topk(M, N, k):
     logits = ext_g[3].cpu()
     G.report("logits", logits, ext_c[3], atol=2e-3, rtol=2e-3) if M <= 2 else None
     rows = [r for r in range(M) if r != 2] if M > 2 else list(range(M))
-    want_p, want_i = torch.softmax(logits[rows], dim=-1).topk(k, dim=-1)
     got_i, got_p = ext_g[4].cpu(), ext_g[5].cpu()
-    # torch.topk does not promise an order among equal values: compare the VALUES picked, and the index rule separately
-    assert torch.equal(torch.gather(logits[rows], 1, got_i[rows]), torch.gather(logits[rows], 1, want_i))
-    torch.testing.assert_close(got_p[rows], want_p, rtol=1e-5, atol=1e-9)
-    key = logits[rows].clone()
-    order = torch.argsort(torch.stack([-key[:, j] for j in range(N)], 1), dim=1, stable=True)[:, :k]   # value desc, index asc
-    if not os.environ.get("VQA_DRY"):          # (the emulator's torch.topk promises no order among equal values)
-        assert torch.equal(got_i[rows], order)
-    if M > 2:                                 # the NaN row: first k indices, NaN probabilities, no fault
-        assert torch.equal(got_i[2], torch.arange(k)) and bool(torch.isnan(got_p[2]).all())
+    if os.environ.get("VQA_DRY"):
+        # the emulator's topk of the probabilities promises no order among equal values or NaN: there only the values
+        # picked in rows with a finite softmax are compared
+        rows = [r for r in rows if not bool(torch.isnan(ref_softmax(logits[r])).any())]
+    order = ref_order(logits[rows], k)
+    torch.testing.assert_close(torch.gather(logits[rows], 1, got_i[rows]), torch.gather(logits[rows], 1, order),
+                               rtol=0, atol=0, equal_nan=True)
+    want_p = torch.gather(ref_softmax(logits[rows]), 1, order).float()
+    torch.testing.assert_close(got_p[rows], want_p, rtol=2e-5, atol=1e-9, equal_nan=True)
     if os.environ.get("VQA_DRY"):
         return
+    assert torch.equal(got_i[rows], order)
+    if M > 2:                                 # the NaN row: first k indices, NaN probabilities, no fault
+        assert torch.equal(got_i[2], torch.arange(k)) and bool(torch.isnan(got_p[2]).all())
+    if special:
+        assert int(torch.isnan(logits[3]).sum()) == 1 and bool(torch.isnan(logits[3, 13]))
+        assert float(logits[4, 17]) == float("inf") and int(torch.isinf(logits[4]).sum()) == 3   # +inf; -inf at 11, 13
+        assert int(got_i[3, 0]) == 13 and int(got_i[4, 0]) == 17
     # replay on the same plan: counters were reset
     from vqa_b200.runtime import Plan
     plan = Plan(gpu.ops, 0)

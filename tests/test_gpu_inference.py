@@ -87,9 +87,12 @@ def test_pipelined_throughput_path_matches_single_calls(engine, lanes, graph):
         assert torch.equal(idx, ridx) and torch.equal(probs, rprobs)
 
 
-@pytest.mark.parametrize("hw", [(300, 400), (100, 160), (333, 211), (224, 500), (640, 224), (17, 23), (1080, 1920), (225, 223)])
+@pytest.mark.parametrize("hw", [(300, 400), (100, 160), (333, 211), (224, 500), (640, 224), (17, 23), (1080, 1920), (225, 223),
+                                (300, 3), (301, 3), (1000, 3), (205, 2), (225, 2), (2000, 5), (70000, 5), (1, 300), (300, 1),
+                                (3000, 4000), (1, 1), (66000, 700)])
 def test_device_resize_is_bit_exact_with_pil(engine, hw):
-    """vqa_resize_bilinear_u8 (csrc/resize.cu) against PIL.Image.resize(BILINEAR) itself: every byte equal."""
+    """vqa_resize_bilinear_u8 (csrc/resize.cu) against PIL.Image.resize(BILINEAR) itself: every byte equal.  (301, 3) ..
+    (70000, 5) take Pillow's vertical-first order (height > 100 * width); 66 000 rows exceed a grid's 65 535 y-blocks."""
     from vqa_b200.runtime import resize_bilinear_u8
     rng = np.random.default_rng(hw[0] * 7919 + hw[1])
     img = rng.integers(0, 256, (hw[0], hw[1], 3), dtype=np.uint8)
@@ -108,6 +111,9 @@ def test_device_resize_matches_golden_and_host_path(engine):
         host = engine.preprocess_image_u8(im, device_resize=False)  # PIL on the host
         assert dev.is_cuda and not host.is_cuda
         assert np.array_equal(dev.cpu().numpy(), g[f"{name}.resized_u8"]) and torch.equal(dev.cpu(), host)
+    tall = Image.fromarray(np.random.default_rng(3).integers(0, 256, (1000, 3, 3), dtype=np.uint8), "RGB")
+    dev = engine.preprocess_image_u8(tall)                          # vertical pass first, as Pillow does
+    assert dev.is_cuda and torch.equal(dev.cpu(), engine.preprocess_image_u8(tall, device_resize=False))
     im = Image.fromarray(g["down.u8"], "RGB")
     engine.gpu_resize = True
     a = engine.predict(im, "what is this", top_k=5)

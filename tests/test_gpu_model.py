@@ -266,10 +266,19 @@ def test_mask_variants_and_padding_invariance(golden_meta):
         b, _ = model(x, t, m.float())
         c, _ = model(x, t, m.int())
         d, _ = model(x, torch.where(m == 0, torch.full_like(t, 17), t), m)
+        e, _ = model(x, t, m.bool())
+        f, _ = model(x, t, m.to(torch.uint8))
         full, _ = model(x, t, None)
         want_full, _ = O.vqa_forward(sd, img, ids, None)
-    assert torch.equal(a, b) and torch.equal(a, c) and torch.equal(a, d)
+    assert torch.equal(a, b) and torch.equal(a, c) and torch.equal(a, d) and torch.equal(a, e) and torch.equal(a, f)
     assert rel_err(full.cpu(), want_full) <= LOGIT_REL_TOL
+    # a uint8 mask is read as weights, like the same values in fp32 (the masked mean pools weigh tokens by the mask)
+    w = mask * (1 + torch.arange(mask.shape[1]) % 3).view(1, -1)       # values 0..3
+    with torch.no_grad():
+        wu, _ = model(x, t, w.to(torch.uint8).cuda())
+        wf, _ = model(x, t, w.float().cuda())
+    assert torch.equal(wu, wf)
+    assert rel_err(wu.cpu(), O.vqa_forward(sd, img, ids, w.float())[0]) <= LOGIT_REL_TOL
 
 
 def test_top1_agreement_10000_pairs():

@@ -56,9 +56,15 @@ def test_no_cpu_path():
         VQAInference(device="cpu").load()
 
 
-@pytest.mark.parametrize("hw", [(300, 400), (100, 160), (333, 211), (224, 500), (640, 224), (17, 23), (225, 223), (1, 1)])
+# (300, 3) .. (2000, 5) and (70000, 5) straddle Pillow's vertical-first rule (height > 100 * width); (1, 300) and
+# (300, 1) are one-pixel strips; (3000, 4000) is a photo-sized downscale.
+RESIZE_SHAPES = [(300, 400), (100, 160), (333, 211), (224, 500), (640, 224), (17, 23), (225, 223), (1, 1),
+                 (300, 3), (301, 3), (1000, 3), (205, 2), (225, 2), (2000, 5), (70000, 5), (1, 300), (300, 1), (3000, 4000)]
+
+
+@pytest.mark.parametrize("hw", RESIZE_SHAPES)
 def test_resize_restatement_is_bit_exact_with_pil(hw):
-    """vqa_b200/resize.py (windows + 22-bit weights handed to the CUDA kernels) and the numpy two-pass
+    """vqa_b200/resize.py (windows + 22-bit weights handed to the CUDA kernels, pass order) and the numpy two-pass
     restatement in oracle/resize_oracle.py against PIL.Image.resize(BILINEAR) itself."""
     from oracle.resize_oracle import numpy_resize
     from vqa_b200.resize import coeffs

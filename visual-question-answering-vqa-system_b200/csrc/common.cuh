@@ -98,6 +98,14 @@ inline cudaError_t vqa_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
+// Rank order of logits shared by every selecting kernel (top-k, accuracy): NaN > +inf > finite > -inf, and equal keys
+// (NaN against NaN, -0.0 against +0.0) go to the lower index.  This is torch.argmax's and torch.topk's order; true when
+// (a, ia) ranks before (b, ib).
+__device__ __forceinline__ bool rank_before(float a, int ia, float b, int ib) {
+  if (a != a) return b == b || ia < ib;
+  return b == b && (a > b || (a == b && ia < ib));
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }

@@ -92,7 +92,7 @@ struct GemmParams {
   // fused softmax + top-k of the output rows (EPI 6: the answer head's last Linear, models/vqa_model.py:336-337):
   // every epilogue thread keeps the running max / exp-sum / k best of its row over the columns it drains and writes them as
   // partial (row, n_tile, column half); the CTA that finishes the last N tile of an M tile (atomic counter) merges them
-  long long* topk_idx;   // [M, topk_k] winners, best first (ties to the lower index, NaN ranks first like torch.topk)
+  long long* topk_idx;   // [M, topk_k] winners, best first (rank_before: ties to the lower index, NaN first like torch.topk)
   float* topk_probs;     // [M, topk_k] softmax probabilities of the winners
   float* topk_part;      // [M, 2 * n_tiles, 2 + 2 * kTopKMax] scratch
   int* topk_cnt;         // [m_tiles] arrival counters (zero between launches: the merging CTA resets its counter)
@@ -133,12 +133,12 @@ __device__ __forceinline__ bool grid_pixel(const GemmParams& p, int row) {
 
 constexpr int kTopKMax = 8;             // fused top-k epilogue: winners kept per thread (larger k: softmax_topk_kernel)
 constexpr int kTopKRec = 4 + 2 * kTopKMax;   // floats per partial record (80 bytes): max, exp-sum, 2 pad, keys, indices
-// (key, index) beats (key', index') when key > key', or on a tie when the index is lower; the list stays sorted best first
+// (key, index) beats (key', index') when it ranks before it (rank_before); the list stays sorted best first
 __device__ __forceinline__ void topk_insert(float (&tv)[kTopKMax], int (&ti)[kTopKMax], float key, int idx) {
-  if (!(key > tv[kTopKMax - 1] || (key == tv[kTopKMax - 1] && idx < ti[kTopKMax - 1]))) return;
+  if (!rank_before(key, idx, tv[kTopKMax - 1], ti[kTopKMax - 1])) return;
 #pragma unroll
   for (int j = kTopKMax - 1; j >= 0; --j) {
-    const bool better = key > tv[j] || (key == tv[j] && idx < ti[j]);
+    const bool better = rank_before(key, idx, tv[j], ti[j]);
     if (better) {
       if (j + 1 < kTopKMax) { tv[j + 1] = tv[j]; ti[j + 1] = ti[j]; }
       tv[j] = key;
@@ -907,7 +907,7 @@ gemm_tap_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant
             }
             if constexpr (kTopK) {
               // online softmax statistics (max ignores NaN like fmaxf, the sum turns NaN like the reference's) and the
-              // k best of the stored values; selection key: NaN ranks above everything (torch.topk's order)
+              // k best of the stored values in rank_before's order (NaN above everything, torch.topk's order)
               float cm = -INFINITY;
 #pragma unroll
               for (int k = 0; k < 32; ++k) {
@@ -925,7 +925,7 @@ gemm_tap_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant
               }
 #pragma unroll
               for (int k = 0; k < 32; ++k) {
-                if (col0 + k < N) topk_insert(tk_v, tk_i, (x[k] != x[k]) ? INFINITY : x[k], col0 + k);
+                if (col0 + k < N) topk_insert(tk_v, tk_i, x[k], col0 + k);
               }
             }
 #pragma unroll

@@ -1466,8 +1466,8 @@ pool_gate_ln_kernel(const float* __restrict__ xatt, const float* __restrict__ te
     reinterpret_cast<__half*>(cat)[static_cast<size_t>(b) * D + d] = __float2half_rn(y);
 }
 
-// softmax over N answers + top-k (k <= 16), ties broken towards the lower index like torch.topk on
-// distinct values (models/vqa_model.py:336-337, api/inference.py:231-234).
+// softmax over N answers + top-k (k <= 128) in rank_before's order, torch.topk's with ties broken towards the lower index
+// (models/vqa_model.py:336-337, api/inference.py:231-234).
 __global__ void softmax_topk_kernel(const float* __restrict__ logits, long long* __restrict__ idx,
                                     float* __restrict__ probs, int N, int k, int ld) {
   pdl_launch_dependents();
@@ -1497,22 +1497,21 @@ __global__ void softmax_topk_kernel(const float* __restrict__ logits, long long*
   s = 0.f;
   for (int w = 0; w < nw; ++w) s += red[w];
   __syncthreads();
-  // Selection key: NaN ranks above everything (torch.topk's order), so a row of NaNs -- the reference's result for a fully
-  // masked question, models/text_encoder.py:244 -- yields indices 0..k-1 with NaN probabilities instead of no winner at
-  // all; a picked entry is retired through the `taken` flag (bit 0 of its key slot), never by its value.
+  // Selection order: NaN ranks above everything (torch.topk's order), so a row of NaNs -- the reference's result for a
+  // fully masked question, models/text_encoder.py:244 -- yields indices 0..k-1 with NaN probabilities instead of no winner
+  // at all; a picked entry is retired through the `taken` flag, never by its value.
   for (int t = 0; t < k; ++t) {
     float best = -INFINITY;
     int bi = 0x7fffffff;
     for (int i = tid; i < N; i += blockDim.x) {
       const float v = vals[i];
-      const float key = (v != v) ? INFINITY : v;
-      if (!taken(i) && (key > best || (key == best && i < bi))) { best = key; bi = i; }
+      if (!taken(i) && rank_before(v, i, best, bi)) { best = v; bi = i; }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const float ob = __shfl_xor_sync(0xffffffffu, best, o);
       const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
+      if (rank_before(ob, oi, best, bi)) { best = ob; bi = oi; }
     }
     if ((tid & 31) == 0) { red[tid >> 5] = best; redi[tid >> 5] = bi; }
     __syncthreads();
@@ -1520,7 +1519,7 @@ __global__ void softmax_topk_kernel(const float* __restrict__ logits, long long*
       float bb = red[0];
       int ii = redi[0];
       for (int w = 1; w < nw; ++w)
-        if (red[w] > bb || (red[w] == bb && redi[w] < ii)) { bb = red[w]; ii = redi[w]; }
+        if (rank_before(red[w], redi[w], bb, ii)) { bb = red[w]; ii = redi[w]; }
       if (ii < 0 || ii >= N) ii = t < N ? t : N - 1;      // cannot happen with k <= N; never index out of the row
       idx[static_cast<size_t>(b) * k + t] = ii;
       probs[static_cast<size_t>(b) * k + t] = expf(vals[ii] - m) / s;

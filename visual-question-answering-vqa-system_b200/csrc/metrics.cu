@@ -5,8 +5,9 @@
 // (training/evaluate.py:77-106, training/train.py:229-264).  Here one kernel per batch ranks the target's logit inside
 // its row and adds to three 64-bit counters that stay in HBM; the host reads them once, in compute().
 //
-// rank(row) = #{ j : v[j] > v[t]  or  (v[j] == v[t] and j < t) }   (t = target; ties go to the lower index, the order
-// argmax / a stable topk pick), so  top-1 correct <=> rank == 0  and  top-k correct <=> rank < k.  A target outside
+// rank(row) = #{ j : v[j] ranks before v[t] }   (t = target; rank_before: NaN > +inf > finite > -inf, ties go to the lower
+// index, the order torch.argmax / torch.topk pick), so  top-1 correct <=> rank == 0  and  top-k correct <=> rank < k, and
+// the predicted index is torch.argmax's (the first NaN of a row that has one).  A target outside
 // [0, N) (AnswerVocabulary.encode returns -1 for unknown answers, data/build_vocab.py:205-218) is never correct and
 // still counts in `total`, exactly as in the reference.  One warp per row; HBM-bound: the logits are read once
 // (4 N bytes per row).
@@ -46,11 +47,14 @@ accuracy_kernel(const float* __restrict__ logits, int ld, int N, const long long
       const float tv = valid ? v[t] : INFINITY;
       const int ti = valid ? static_cast<int>(t) : -1;
       int above = 0;
-      float best = -INFINITY;
+      float best = -INFINITY, special = 0.f;
       int bi = 0x7fffffff;
+      // the streaming pass compares as for finite rows and only notes whether the row holds a NaN or an infinity
+      // (x * 0 is NaN then): comparing every element with rank_before here halved the achieved bandwidth
       auto visit = [&](float x, int j) {
         above += (x > tv || (x == tv && j < ti)) ? 1 : 0;
         if (x > best || (x == best && j < bi)) { best = x; bi = j; }
+        special = fmaf(x, 0.f, special);
       };
       if (((reinterpret_cast<uintptr_t>(v) | (static_cast<uintptr_t>(ld) * 4)) & 15) == 0) {
         // 16-byte loads (row pitch and base aligned): 512 bytes per warp instruction, two in flight per lane
@@ -71,12 +75,23 @@ accuracy_kernel(const float* __restrict__ logits, int ld, int N, const long long
 #pragma unroll 8
         for (int j = lane; j < N; j += 32) visit(v[j], j);
       }
+      if (__any_sync(0xffffffffu, special != special)) {
+        // a NaN or an infinity in the row: recount it in rank_before's order (the row is read a second time)
+        above = 0;
+        best = -INFINITY;
+        bi = 0x7fffffff;
+        for (int j = lane; j < N; j += 32) {
+          const float x = v[j];
+          above += rank_before(x, j, tv, ti) ? 1 : 0;
+          if (rank_before(x, j, best, bi)) { best = x; bi = j; }
+        }
+      }
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) {
         above += __shfl_xor_sync(0xffffffffu, above, o);
         const float ob = __shfl_xor_sync(0xffffffffu, best, o);
         const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-        if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
+        if (rank_before(ob, oi, best, bi)) { best = ob; bi = oi; }
       }
       if (lane == 0) {
         if (valid && above == 0) atomicAdd(&s_top1, 1u);

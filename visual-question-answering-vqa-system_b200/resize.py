@@ -5,7 +5,10 @@ The reference resizes through ``torchvision.transforms.Resize((224, 224))`` on P
 Pillow is a third-party dependency of the reference (``Pillow>=9.5.0`` in requirements.txt; 12.2.0 in this
 image; C source ``src/libImaging/Resample.c`` is not vendored), so its published algorithm is restated here:
 
-* separable, horizontal pass first, then vertical; the intermediate image is rounded to uint8;
+* separable, horizontal pass first, then vertical; the intermediate image is rounded to uint8.  An image more than
+  100 times taller than wide that shrinks vertically goes vertical pass first (``vertical_first``): the installed
+  Pillow (12.2.0) does so in ``Image.resize``, earlier releases always ran horizontal first, and this module follows
+  the installed one;
 * triangle filter with support ``max(scale, 1)``; per output pixel a window ``[xmin, xmin + n)`` with
   ``xmin = int(center - support + 0.5)``, weights normalised to sum 1 in double precision;
 * 8-bit path: weights become 22-bit fixed point (round half away from zero), each output is
@@ -24,6 +27,12 @@ from typing import Tuple
 import numpy as np
 
 PRECISION_BITS = 32 - 8 - 2
+
+
+def vertical_first(in_h: int, in_w: int, out_h: int) -> bool:
+    """Pass order of ``Image.resize``: True when Pillow resizes rows before columns (``in_h > 100 * in_w`` and the
+    height shrinks).  The two orders round the intermediate image differently, so they give different bytes."""
+    return in_h > in_w * 100 and out_h < in_h
 
 
 @lru_cache(maxsize=256)

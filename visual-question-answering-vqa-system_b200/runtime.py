@@ -129,9 +129,10 @@ class Plan:
 
 
 def resize_bilinear_u8(src, out_h: int = 224, out_w: int = 224, stream=None):
-    """PIL-exact antialiased bilinear resize of one uint8 HWC CUDA tensor (``vqa_resize_bilinear_u8``)."""
+    """PIL-exact antialiased bilinear resize of one uint8 HWC CUDA tensor (``vqa_resize_bilinear_u8``), in Pillow's pass
+    order (``resize.vertical_first``: vertical first is two single-pass calls through an intermediate image)."""
     import torch
-    from .resize import coeffs
+    from .resize import coeffs, vertical_first
     if src.device.type != "cuda" or src.dtype != torch.uint8 or src.dim() != 3:
         raise VqaError("resize_bilinear_u8 expects a uint8 [H, W, C] CUDA tensor (there is no CPU path)")
     src = src.contiguous()
@@ -140,22 +141,34 @@ def resize_bilinear_u8(src, out_h: int = 224, out_w: int = 224, stream=None):
     st = stream if stream is not None else torch.cuda.current_stream(dev)
     dst = torch.empty(out_h, out_w, ch, dtype=torch.uint8, device=dev)
     ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
-    bh = kh = bv = kv = tmp = None
-    ksh = ksv = 0
-    with torch.cuda.stream(st):
-        if in_w != out_w:
-            b, k = coeffs(in_w, out_w)
-            bh, kh, ksh = torch.from_numpy(b).to(dev), torch.from_numpy(k).to(dev), k.shape[1]
-        if in_h != out_h:
-            b, k = coeffs(in_h, out_h)
-            bv, kv, ksv = torch.from_numpy(b).to(dev), torch.from_numpy(k).to(dev), k.shape[1]
-        if in_w != out_w and in_h != out_h:
-            tmp = torch.empty(in_h, out_w, ch, dtype=torch.uint8, device=dev)
-        check(lib().vqa_resize_bilinear_u8(ptr(src), in_h, in_w, ch, ptr(tmp), ptr(dst), out_h, out_w, ptr(bh), ptr(kh), ksh,
+    keep = [src]
+
+    def call(a, a_h, a_w, b, b_h, b_w, tmp=None):
+        bh = kh = bv = kv = None
+        ksh = ksv = 0
+        if a_w != b_w:
+            bnd, k = coeffs(a_w, b_w)
+            bh, kh, ksh = torch.from_numpy(bnd).to(dev), torch.from_numpy(k).to(dev), k.shape[1]
+        if a_h != b_h:
+            bnd, k = coeffs(a_h, b_h)
+            bv, kv, ksv = torch.from_numpy(bnd).to(dev), torch.from_numpy(k).to(dev), k.shape[1]
+        check(lib().vqa_resize_bilinear_u8(ptr(a), a_h, a_w, ch, ptr(tmp), ptr(b), b_h, b_w, ptr(bh), ptr(kh), ksh,
                                            ptr(bv), ptr(kv), ksv, C.c_void_p(st.cuda_stream)))
-        for t in (src, tmp, bh, kh, bv, kv):
-            if t is not None:
-                t.record_stream(st)
+        keep.extend(t for t in (tmp, bh, kh, bv, kv) if t is not None)
+
+    with torch.cuda.stream(st):
+        if in_w != out_w and in_h != out_h:
+            if vertical_first(in_h, in_w, out_h):
+                mid = torch.empty(out_h, in_w, ch, dtype=torch.uint8, device=dev)
+                call(src, in_h, in_w, mid, out_h, in_w)
+                call(mid, out_h, in_w, dst, out_h, out_w)
+                keep.append(mid)
+            else:
+                call(src, in_h, in_w, dst, out_h, out_w, tmp=torch.empty(in_h, out_w, ch, dtype=torch.uint8, device=dev))
+        else:
+            call(src, in_h, in_w, dst, out_h, out_w)
+        for t in keep:
+            t.record_stream(st)
     return dst
 
 
