@@ -12,6 +12,7 @@ import math
 import torch
 import torch.nn.functional as F
 
+import topk_ref as TR
 from vqa_b200 import program as P
 
 MEAN = torch.tensor([0.485, 0.456, 0.406])
@@ -405,8 +406,13 @@ class Emulator:
         if op.p.get("mask") is not None:
             mask = _t(op.p["mask"], torch.int32, ext)[: B * L].view(B, L)
         ctx, _ = self._attend(q, k, v, hd, mask)
-        odt = torch.float16 if i.get("no_round") == 2 else torch.float32
-        _t(op.p["out"], odt, ext)[: B * L * D].view(B, L, D).copy_(ctx.transpose(1, 2).reshape(B, L, D).to(odt))
+        self._attn_store(op.p["out"], i.get("no_round", 0), ctx.transpose(1, 2).reshape(B, L, D), ext)
+
+    @staticmethod
+    def _attn_store(ref, no_round, ctx, ext):
+        """Attention output forms: 2 = fp16, 1 = fp32, 0 = tf32-rounded fp32."""
+        odt = torch.float16 if no_round == 2 else torch.float32
+        _t(ref, odt, ext)[: ctx.numel()].view(ctx.shape).copy_(ctx.to(odt) if no_round else P.round_tf32(ctx))
 
     def op_cross_attn(self, op, ext):
         i = op.i
@@ -420,8 +426,7 @@ class Emulator:
         v = torch.as_strided(kvf[i["v_off"]:], (Bi * T, D), (i["ld_kv"], 1)).view(Bi, T, H, hd).transpose(1, 2)
         k, v = k.repeat_interleave(qk, dim=0), v.repeat_interleave(qk, dim=0)
         ctx, w = self._attend(q, k, v, hd)
-        odt = torch.float16 if i.get("no_round") == 2 else torch.float32
-        _t(op.p["out"], odt, ext)[: B * L * D].view(B, L, D).copy_(ctx.transpose(1, 2).reshape(B, L, D).to(odt))
+        self._attn_store(op.p["out"], i.get("no_round", 0), ctx.transpose(1, 2).reshape(B, L, D), ext)
         if op.p.get("weights") is not None:
             _t(op.p["weights"], torch.float32, ext)[: B * H * L * T].view(B, H, L, T).copy_(w)
 
@@ -465,6 +470,9 @@ class Emulator:
         B, N, k = i["B"], i["N"], i["k"]
         logits = torch.as_strided(ext[op.p["logits"].slot].view(-1), (B, N), (i["ld"], 1))
         probs, idx = F.softmax(logits, dim=-1).topk(k, dim=-1)
+        nan_rows = torch.isnan(logits).any(dim=1)
+        if bool(nan_rows.any()):                 # the kernel's order: NaN ties go to the lower index
+            idx[nan_rows] = TR.ref_order(logits[nan_rows], k)
         ext[op.p["idx"].slot].view(B, k).copy_(idx)
         ext[op.p["probs"].slot].view(B, k).copy_(probs)
 

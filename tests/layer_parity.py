@@ -18,6 +18,7 @@ from typing import Callable, List, Optional
 import torch
 
 import emulator as E
+import topk_ref as TR
 from oracle import vqa_oracle as O
 from vqa_b200 import program as P
 from vqa_b200.model import VQAModel
@@ -177,11 +178,14 @@ def _where(idx, shape, labels, index_map=None):
 class Checker:
     """Walks ``prog`` with ``runner(first, last)`` (runs ops [first, last) and returns when they are done) and compares
     every module with its fp64 reference.  ``imgs``: the images whose backbone layers are checked (default all); pads,
-    projector, K/V and the whole text / fusion / head side are checked for every image and pair."""
+    projector, K/V and the whole text / fusion / head side are checked for every image and pair.
+    ``image_projected``: for a question-side program (side="question", K/V from the image cache), the projected image
+    tokens [n_images, 49, D] of the image-side program that made the cache; the cross layers' references use them."""
 
     def __init__(self, prog: P.Program, sd, ext, runner: Callable[[int, int], None], imgs=None,
-                 kernel_name: Optional[Callable[[int], str]] = None, title: str = ""):
+                 kernel_name: Optional[Callable[[int], str]] = None, title: str = "", image_projected=None):
         self.prog, self.ext, self.runner = prog, ext, runner
+        self.image_projected = None if image_projected is None else image_projected.to(prog.ws.tensor.device, torch.float64)
         self.dev = prog.ws.tensor.device
         self.sd = {k: v.detach().to(self.dev, torch.float64) for k, v in sd.items()}
         self.cfg = prog.cfg
@@ -208,11 +212,19 @@ class Checker:
     def _cmp(self, module, output, cls, got, want, labels, at, index_map=None, chan=False):
         got, want = got.to(torch.float64), want.to(torch.float64)
         assert got.shape == want.shape, (module, output, tuple(got.shape), tuple(want.shape))
+        nan_ref = torch.isnan(want)
+        if bool(nan_ref.any()):
+            # a fully masked question is NaN in the reference (SURVEY T5): the output must be NaN at exactly those
+            # elements (an element that is not counts as an infinite error) and is compared as usual everywhere else
+            got = torch.where(nan_ref, torch.where(torch.isnan(got), 0.0, math.inf), got)
+            want = torch.where(nan_ref, 0.0, want)
         d = got - want
         err = d.abs()
         amax = float(want.abs().max())
         k = int(torch.nan_to_num(err, nan=math.inf).argmax())
         rms_ref = float(want.pow(2).mean().sqrt())
+        if amax == 0.0 and bool(nan_ref.all()):        # NaN everywhere in the reference: no finite element to scale by
+            amax = rms_ref = 1.0
         row = Row(module, output, cls, float(err.max()) / amax, float(err.pow(2).mean().sqrt()) / rms_ref,
                   _where(k, got.shape, labels, index_map), GATES[self.mode][cls], kernel=self.kernel_name(at))
         if chan:
@@ -380,7 +392,10 @@ class Checker:
 
             def cross(l=l, kl=kl, q_name=q_name):
                 q_in = self.snaps.pop("x.q") if q_name == "x.q" else tokens(prog, "text_features", B, L)
-                img = prog.tensor("image_projected").view(Bi, 49, -1).to(torch.float64).repeat_interleave(B // Bi, dim=0)
+                img = self.image_projected
+                if img is None:
+                    img = prog.tensor("image_projected").view(Bi, 49, -1).to(torch.float64)
+                img = img.repeat_interleave(B // Bi, dim=0)
                 want, w = O.cross_layer(sd, f"fusion.cross_attention.layers.{l}", q_in, img, self.heads)
                 self.snaps["x.q"] = tokens(prog, "x.q", B, L)
                 self._cmp(f"x.{l}", "x.q", "linear", self.snaps["x.q"], want, tok, kl)
@@ -410,6 +425,9 @@ class Checker:
 
             def topk():
                 wi, wp = O.predict_topk(logits.to(torch.float64), prog.top_k)
+                nan_rows = torch.isnan(logits).any(dim=1)
+                if bool(nan_rows.any()):          # torch.topk orders NaN ties arbitrarily; the kernels take lower indices first
+                    wi[nan_rows] = TR.ref_order(logits[nan_rows], prog.top_k).to(wi.device)
                 gi, gp = ext[P.EXT["top_idx"]], ext[P.EXT["top_probs"]]
                 bad = (gi != wi).any(dim=1)
                 first = int(bad.nonzero()[0]) if bool(bad.any()) else -1
@@ -442,25 +460,41 @@ ABLATE = dict(use_se_attention=False, use_spatial_attention=False, use_gating=Fa
 NOSPATIAL = dict(use_spatial_attention=False)
 
 
+MASK_CODES = {torch.int64: P.MASK_I64, torch.float32: P.MASK_F32, torch.int32: P.MASK_I32, torch.bool: P.MASK_U8,
+              torch.uint8: P.MASK_U8}     # what Engine passes for each attention_mask dtype
+
+
 def make_case(ctor, B, L=None, in_fmt="nchw_f32", mask_kind="i64", precision="bf16", window=True, n_images=None,
-              device="cpu", seed=1234, top_k=5):
+              device="cpu", seed=1234, top_k=5, ids=None, mask=None, side="both"):
     """A seeded model (randomised BN / LayerNorm state), its program on ``device`` and the external slots.
-    Returns (prog, sd, ext)."""
+    ``ids`` / ``mask`` [B, L]: explicit questions instead of the seeded ones; the mask's dtype (int64, float32, int32,
+    bool, uint8) then selects the mask code and ``mask_kind`` is ignored.  side="question": the question side only, its
+    cross-attention K/V read from the slots ext[P.EXT["kv{l}"]], which the caller fills.  Returns (prog, sd, ext)."""
     torch.manual_seed(0)
     model = VQAModel(**ctor).eval()
     sd = randomise_state(model.state_dict(), 1)
     cfg = model.config
-    L = L or cfg["max_question_length"]
+    L = L or (ids.shape[1] if ids is not None else cfg["max_question_length"])
     Bi = B if n_images is None else n_images
-    u8, img, ids, mask = synth_batch(B, seed, max_len=L, vocab=cfg["vocab_size"])
+    u8, img, sids, smask = synth_batch(B, seed, max_len=L, vocab=cfg["vocab_size"])
     images = (u8 if in_fmt == "hwc_u8" else img)[:Bi]
-    code = {"i64": P.MASK_I64, "f32": P.MASK_F32, "none": P.MASK_NONE}[mask_kind]
-    m = {"i64": mask, "f32": mask.float(), "none": None}[mask_kind]
+    if ids is None:
+        ids = sids
+    assert tuple(ids.shape) == (B, L) and ids.dtype == torch.int64
+    if mask is not None:
+        assert tuple(mask.shape) == (B, L)
+        code, m = MASK_CODES[mask.dtype], mask
+    else:
+        code = {"i64": P.MASK_I64, "f32": P.MASK_F32, "none": P.MASK_NONE}[mask_kind]
+        m = {"i64": smask, "f32": smask.float(), "none": None}[mask_kind]
     W = P.build_weights(sd, cfg, device, precision=precision)
-    prog = P.Program(W, cfg, B, L, in_fmt, code, want_aux=True, top_k=top_k, device=device, window=window, n_images=n_images)
+    prog = P.Program(W, cfg, B, L, in_fmt, code, want_aux=side == "both", top_k=top_k, device=device, window=window,
+                     n_images=n_images, side=side)
     NA = cfg["num_answers"]
     ext = [images, ids, m, torch.zeros(B, NA), torch.zeros(B, max(top_k, 1), dtype=torch.int64), torch.zeros(B, max(top_k, 1))]
     ext = [None if t is None else t.to(device) for t in ext]
+    if side == "question":
+        ext += [None] * (len(P.EXT) - len(ext))
     return prog, sd, ext
 
 
@@ -469,5 +503,6 @@ def emulator_runner(prog, ext):
     return lambda first, last: emu.run(ext, first, last)
 
 
-def check_on_emulator(prog, sd, ext, imgs=None, title="") -> Report:
-    return Checker(prog, sd, ext, emulator_runner(prog, ext), imgs=imgs, kernel_name=lambda k: "", title=title).run()
+def check_on_emulator(prog, sd, ext, imgs=None, title="", image_projected=None) -> Report:
+    return Checker(prog, sd, ext, emulator_runner(prog, ext), imgs=imgs, kernel_name=lambda k: "", title=title,
+                   image_projected=image_projected).run()

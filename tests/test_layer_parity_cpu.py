@@ -67,6 +67,32 @@ def _shift_key_mask(prog):
     op.p["mask"] = P.Buf(m.arena, m.offset + 4, m.nbytes, m.name)
 
 
+def _empty_question_case():
+    """Three questions of 20 tokens; the second is fully masked, which the reference turns into NaN (SURVEY T5)."""
+    mask = torch.ones(3, 20, dtype=torch.int64)
+    mask[1] = 0
+    mask[2, 5:] = 0
+    return LP.make_case({}, B=3, mask=mask)
+
+
+def test_checker_matches_nan_positions():
+    """Where the fp64 reference is NaN the program must be NaN at exactly those elements; a key mask read one question
+    to the left moves the NaN to another question, and the checker charges that to the first encoder layer only."""
+    prog, sd, ext = _empty_question_case()
+    rep = LP.check_on_emulator(prog, sd, ext, title="fully masked question")
+    assert not rep.failures(), rep.table()
+    logits = ext[P.EXT["logits"]]
+    assert bool(torch.isnan(logits[1]).all()) and not bool(torch.isnan(logits[[0, 2]]).any())
+
+    prog, sd, ext = _empty_question_case()
+    op = _op(prog, "text.0.attn")
+    m = op.p["mask"]
+    op.p["mask"] = P.Buf(m.arena, m.offset + 4 * prog.L, m.nbytes, m.name)
+    rep = LP.check_on_emulator(prog, sd, ext, title="key mask shifted by one question")
+    print(rep.table())
+    assert rep.failing_modules() == ["text.0"], rep.table()
+
+
 @pytest.mark.parametrize("mutate,module", [
     (_swap_taps, "s3.b0.conv1"),
     (_mask_last_row, "s3.b0.conv1"),

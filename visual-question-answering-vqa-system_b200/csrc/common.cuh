@@ -341,6 +341,10 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   return *reinterpret_cast<uint32_t*>(&v);
 }
 
+// ReLU that keeps NaN, as torch.relu and the cvt.relu packs below do (fmaxf(NaN, 0) is 0: a fully masked question's NaN
+// would turn into finite logits)
+__device__ __forceinline__ float relu_f32(float x) { return x != x ? x : fmaxf(x, 0.f); }
+
 // max(x, 0) rounded to bf16 (RN) in one instruction per pair
 __device__ __forceinline__ uint32_t pack_relu_bf16x2(float lo, float hi) {
   uint32_t d;

@@ -888,14 +888,14 @@ gemm_tap_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant
             if (sums != nullptr) {                      // SE squeeze partial sums of this 32-row slab (warp-uniform branch)
               const bool live = pix[sub] && row0 + lane < p.M;     // rows past M exist only in the accumulator
 #pragma unroll
-              for (int k = 0; k < 32; ++k) x[k] = live ? (relu ? fmaxf(x[k], 0.f) : x[k]) : 0.f;
+              for (int k = 0; k < 32; ++k) x[k] = live ? (relu ? relu_f32(x[k]) : x[k]) : 0.f;
               const float tot = warp_colsum32(x, lane);
               if (row0 < p.M && col0 + lane < N) sums[static_cast<size_t>(row0 >> 5) * ld_sums + col0 + lane] = tot;
             }
           } else {
             if (relu) {
 #pragma unroll
-              for (int k = 0; k < 32; ++k) x[k] = fmaxf(x[k], 0.f);
+              for (int k = 0; k < 32; ++k) x[k] = relu_f32(x[k]);
             }
             if (!pix[sub]) {
 #pragma unroll
