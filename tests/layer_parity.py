@@ -18,6 +18,7 @@ from typing import Callable, List, Optional
 import torch
 
 import emulator as E
+import schedule as S
 import topk_ref as TR
 from oracle import vqa_oracle as O
 from vqa_b200 import program as P
@@ -496,6 +497,18 @@ def make_case(ctor, B, L=None, in_fmt="nchw_f32", mask_kind="i64", precision="bf
     if side == "question":
         ext += [None] * (len(P.EXT) - len(ext))
     return prog, sd, ext
+
+
+def poison(prog):
+    """Fill the workspace with 0xFF bytes (NaN in fp32, bf16 and fp16), the gaps between allocations and the trailing
+    slack included, and give back their zeros to the regions a run reads without writing (``schedule.ALLOW``).  A module
+    then passes only if its producers wrote every byte it reads, pads included.  Poison is data only: the workspace's
+    integer buffers are the key mask, which the embedding / mask op writes before any use, and the allow-listed top-k
+    counters, so nothing a kernel uses as an address or an index is poisoned."""
+    ws = prog.ws.tensor
+    ws.fill_(0xFF)
+    for lo, hi in S.allowed_ranges(prog):
+        ws[lo:hi] = 0
 
 
 def emulator_runner(prog, ext):

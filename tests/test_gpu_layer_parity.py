@@ -2,7 +2,8 @@
 forward -- ingest, stem, each convolution, each block output, each stage tail with its SE scale and spatial map, the
 projector, each K/V projection, the embedding, each text layer, the final norm, each cross layer with its attention
 weights, pools / gate / output norm, head and top-k -- against an fp64 restatement of its reference module applied to
-the module's own inputs as the GPU left them, plus every pad cell of every padded-flat grid exactly 0.
+the module's own inputs as the GPU left them, plus every pad cell of every padded-flat grid exactly 0.  The workspace is
+filled with 0xFF bytes before each walk (``layer_parity.poison``), so a pad cell is 0 only if its producer wrote it.
 
 The fp64 references run on the same device (torch, fp64), one module at a time between op ranges of the plan; the whole
 file takes about 15 s on a B200.  Worst max|err| / max|ref| measured on B200 (1000 W), per class:
@@ -28,6 +29,7 @@ DEV = "cpu" if DRY else "cuda"
 
 
 def _check(prog, sd, ext, imgs=None, title=""):
+    LP.poison(prog)              # the pad checks then prove that the pads were written
     if DRY:
         rep = LP.check_on_emulator(prog, sd, ext, imgs=imgs, title=title)
     else:

@@ -1023,7 +1023,8 @@ class Program(OpList):
         xn = self._buf("text.xn", self.tdt, T, D)
         qkv = self._buf("text.qkv", f32, T, 3 * D)
         ctx = self._buf("text.ctx", self.tdt, T, D)
-        hid = self._buf("text.hid", self.tdt, T, F)
+        chain = self.chain and D == 256 and F % 128 == 0 and F <= 1024
+        hid = None if chain else self._buf("text.hid", self.tdt, T, F)    # the chain kernels keep the FFN hidden state on chip
         V = W.items["text.emb"][2][0]
         if fuse_embed:   # embedding + position, the first layer's LayerNorm and the mask normalisation in one launch
             self._op("embed", "text.embed", dict(B=B, L=L, D=D, V=V, round_tf32=self._ln_mode(True), mask_dtype=self.mask_dtype),
@@ -1035,7 +1036,6 @@ class Program(OpList):
             self._op("embed", "text.embed", dict(B=B, L=L, D=D, V=V),
                      dict(ids=ExtRef(EXT["ids"]), table=W.buf("text.emb"), pe=W.buf("text.pe"), dst=xt))
         layer = 0
-        chain = self.chain and D == 256 and F % 128 == 0 and F <= 1024
         while f"text.{layer}.qkv.w" in W:
             p = f"text.{layer}"
             if not (chain and layer > 0):         # chains: the previous layer's kernel already produced this layer's q, k, v
@@ -1068,7 +1068,7 @@ class Program(OpList):
         # side lane right before each attention.  Ops are issued in list order, so a JOIN waits only for what
         # precedes it in the list.
         q = self._buf("x.q", f32, T, D)          # running query (residual stream)
-        qn = self._buf("x.qn", self.tdt, T, D)
+        qn = None if chain else self._buf("x.qn", self.tdt, T, D)   # chains: each layer's kernel normalises the next query
         qp = self._buf("x.qp", f32, T, D)
         cx = self._buf("x.ctx", self.tdt, T, D)
         if cached:
