@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define VQA_ABI_VERSION 9
+#define VQA_ABI_VERSION 10
 
 #define VQA_OK            0
 #define VQA_E_INVALID    -1   /* bad argument / unsupported shape */
@@ -81,7 +81,10 @@ enum VqaOpKind {
                                 per N = 128 MMA, vertical max carried in registers along runs of pooled rows */
   VQA_OP_MLP_CHAIN     = 20, /* fused post-attention chain of a transformer layer: W_o + residual, LayerNorm, FFN, residual and the next
                                 block's LayerNorm + projection (models/text_encoder.py:373-399, models/cross_attention.py:265-299) */
-  VQA_OP_KIND_MAX      = 21
+  VQA_OP_ATTN_CHUNKED  = 21, /* masked softmax(QK^T/sqrt(d))V with the keys streamed in chunks of 64 (online softmax): the self-
+                                (models/text_encoder.py:229-259) and cross-attention (models/cross_attention.py:164-197) of
+                                questions longer than 64 tokens, up to 512 queries and 512 keys */
+  VQA_OP_KIND_MAX      = 22
 };
 
 typedef struct VqaOp {

@@ -1195,6 +1195,16 @@ __device__ __forceinline__ void mma_3xtf32(float (&d)[4], const uint32_t (&ah)[4
   mma_tf32(d, ah, bh0, bh1);
 }
 
+// Two adjacent context values (element e of out) in the form of W_o's operand: fp16 (2), unrounded for the 3xTF32
+// split (1), tf32 (0).
+__device__ __forceinline__ void attn_store2(float* out, size_t e, int no_round, float o0, float o1) {
+  if (no_round == 2) {
+    *reinterpret_cast<uint32_t*>(reinterpret_cast<__half*>(out) + e) = pack_f16x2(o0, o1);
+  } else {
+    *reinterpret_cast<float2*>(out + e) = no_round ? make_float2(o0, o1) : make_float2(round_tf32_rna(o0), round_tf32_rna(o1));
+  }
+}
+
 constexpr int kKs = 36, kVs = 40;                       // padded row strides (floats): conflict-free fragment loads
 __host__ __device__ constexpr int attn_mma_kreg(int nt) {           // K rows, later the probability tile [32][nt*8+4]
   return nt * 8 * kKs > 32 * (nt * 8 + 4) ? nt * 8 * kKs : 32 * (nt * 8 + 4);
@@ -1348,18 +1358,9 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
       for (int hf = 0; hf < 2; ++hf) {
         const int row = l0 + mt * 16 + hf * 8 + g;
         if (row < L) {
-          float* orow = out + (static_cast<size_t>(b) * L + row) * (H * kHd) + h * kHd + 2 * t;
+          const size_t e0 = (static_cast<size_t>(b) * L + row) * (H * kHd) + h * kHd + 2 * t;
 #pragma unroll
-          for (int n = 0; n < 4; ++n) {                 // operand of W_o: fp16 (2), unrounded for the 3xTF32 split (1), tf32 (0)
-            const float o0 = oacc[mt][n][hf * 2], o1 = oacc[mt][n][hf * 2 + 1];
-            if (no_round == 2) {
-              __half* hrow = reinterpret_cast<__half*>(out) + (static_cast<size_t>(b) * L + row) * (H * kHd) + h * kHd + 2 * t;
-              *reinterpret_cast<uint32_t*>(hrow + n * 8) = pack_f16x2(o0, o1);
-            } else {
-              *reinterpret_cast<float2*>(orow + n * 8) = no_round ? make_float2(o0, o1)
-                                                                  : make_float2(round_tf32_rna(o0), round_tf32_rna(o1));
-            }
-          }
+          for (int n = 0; n < 4; ++n) attn_store2(out, e0 + n * 8, no_round, oacc[mt][n][hf * 2], oacc[mt][n][hf * 2 + 1]);
         }
       }
   }
@@ -1389,6 +1390,235 @@ static int launch_attn(const float* q, const float* k, const float* v, const int
   VQA_CUDA_OK(vqa_launch(fn, dim3((B * H + kAttnWarps - 1) / kAttnWarps), dim3(kAttnWarps * 32), smem, st, q, k, v, mask, out,
                          weights, B * H, H, L, T, ld_q, ld_kv, no_round, q_per_kv));
   VQA_LAUNCH_OK("attn_mma_kernel");
+  return VQA_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Attention with the keys streamed in chunks of 64, for questions longer than 64 tokens: up to 512 queries and 512
+// keys, otherwise the arithmetic of attn_mma_kernel (3xTF32 mma.sync for S = Q K^T and O = P V, fp32 softmax, the same
+// fragment layouts and output forms).  attn_mma_kernel keeps all keys of a (pair, head) in one warp and stays the
+// kernel of questions of at most 64 tokens (program.py::ATTN_MMA_MAX_L; DESIGN.md, "Long questions").
+// A CTA of up to 4 warps covers (pair, head, up to 128 queries), 32 queries per warp; its warps share double-buffered
+// 64-key K / V chunks that cp.async brings into shared memory while the previous chunk is consumed.
+// Online softmax: per query row a running max m, a running sum l and the context accumulator, rescaled by exp(m_old -
+// m_new) at every chunk.  While every key seen so far is masked the max used in exp() is 0 instead of -inf, so a chunk
+// of only masked keys adds exactly nothing (rather than exp(-inf - -inf) = NaN) and a row that has a valid key anywhere
+// is finite.  A row whose keys are all masked ends with l = 0 and a zero accumulator: 0 * (1 / 0) = NaN at every
+// element, as in the reference (SURVEY T5).
+constexpr int kChunk = 64;                               // keys per chunk (8 tiles of 8)
+constexpr int kCkWarps = 4;
+constexpr int kCkStage = kChunk * (kKs + kVs);           // floats of one K + V chunk
+constexpr int kCkPS = kChunk + 4;                        // probability tile row stride
+constexpr int kCkSmemFloats = 2 * kCkStage + 2 * kChunk + kCkWarps * 32 * kCkPS;   // K/V x 2, key flags x 2, P per warp
+
+__global__ void __launch_bounds__(kCkWarps * 32)
+attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v,
+                    const int* __restrict__ mask, float* __restrict__ out, float* __restrict__ weights, int H, int L, int T,
+                    int ld_q, int ld_kv, int no_round, int q_per_kv) {
+  pdl_launch_dependents();
+  pdl_wait();
+  extern __shared__ __align__(16) float sm[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+  const int g = lane >> 2, t = lane & 3;
+  const int unit = blockIdx.x;                          // (pair, head)
+  const int b = unit / H, h = unit - b * H;
+  const int l0 = (blockIdx.y * nw + warp) * 32;         // this warp's first query
+  const bool active = l0 < L;
+  int* flags = reinterpret_cast<int*>(sm + 2 * kCkStage);   // [2][kChunk]: 1 = a valid key
+  float* Ps = sm + 2 * kCkStage + 2 * kChunk + warp * 32 * kCkPS;
+  const float* qb = q + static_cast<size_t>(b) * L * ld_q + h * kHd;
+  const int bkv = b / q_per_kv;                         // q_per_kv consecutive queries share one image's K / V
+  const float* kb = k + static_cast<size_t>(bkv) * T * ld_kv + h * kHd;
+  const float* vb = v + static_cast<size_t>(bkv) * T * ld_kv + h * kHd;
+  const int n_chunks = (T + kChunk - 1) / kChunk;
+  // chunk c -> stage c & 1: K and V rows (rows beyond T zero-filled through the src-size operand) and the key flags
+  auto stage = [&](int c) {
+    float* Ks = sm + (c & 1) * kCkStage;
+    float* Vs = Ks + kChunk * kKs;
+    for (int i = threadIdx.x; i < kChunk * 8; i += blockDim.x) {
+      const int r = i >> 3, c4 = i & 7, j = c * kChunk + r;
+      const size_t off = static_cast<size_t>(j < T ? j : 0) * ld_kv + c4 * 4;
+      const uint32_t dk = static_cast<uint32_t>(__cvta_generic_to_shared(Ks + r * kKs + c4 * 4));
+      const uint32_t dv = static_cast<uint32_t>(__cvta_generic_to_shared(Vs + r * kVs + c4 * 4));
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dk), "l"(kb + off), "r"(j < T ? 16 : 0) : "memory");
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dv), "l"(vb + off), "r"(j < T ? 16 : 0) : "memory");
+    }
+    for (int r = threadIdx.x; r < kChunk; r += blockDim.x) {
+      const int j = c * kChunk + r;
+      flags[(c & 1) * kChunk + r] = j < T && (mask == nullptr || mask[static_cast<size_t>(b) * T + j] != 0);
+    }
+    asm volatile("cp.async.commit_group;" ::: "memory");
+  };
+  stage(0);
+  // Q fragments (rows g, g+8 of each 16-row tile; dims t, t+4 of each 8-wide k step), pre-split
+  uint32_t qh[2][4][4], ql[2][4][4];
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int ks = 0; ks < 4; ++ks)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const int row = l0 + mt * 16 + g + (e & 1) * 8, col = ks * 8 + t + (e >> 1) * 4;
+        const float x = row < L ? __ldg(qb + static_cast<size_t>(row) * ld_q + col) : 0.f;
+        split_tf32(x, qh[mt][ks][e], ql[mt][ks][e]);
+      }
+  const float scale = rsqrtf(static_cast<float>(kHd));
+  float m_run[2][2], l_run[2][2], oacc[2][4][4];        // per (16-row tile, row half): running max / sum
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int hf = 0; hf < 2; ++hf) {
+      m_run[mt][hf] = -INFINITY;
+      l_run[mt][hf] = 0.f;
+    }
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int n = 0; n < 4; ++n)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) oacc[mt][n][e] = 0.f;
+
+  for (int c = 0; c < n_chunks; ++c) {
+    if (c + 1 < n_chunks) {
+      stage(c + 1);                                     // its stage was released by the barrier that ended chunk c - 1
+      asm volatile("cp.async.wait_group 1;" ::: "memory");
+    } else {
+      asm volatile("cp.async.wait_group 0;" ::: "memory");
+    }
+    __syncthreads();                                    // chunk c has landed, from every thread's copies
+    if (active) {
+      const float* Ks = sm + (c & 1) * kCkStage;
+      const float* Vs = Ks + kChunk * kKs;
+      const int* fl = flags + (c & 1) * kChunk;
+      float sacc[2][8][4];
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int n = 0; n < 8; ++n)
+#pragma unroll
+          for (int e = 0; e < 4; ++e) sacc[mt][n][e] = 0.f;
+#pragma unroll
+      for (int ks = 0; ks < 4; ++ks)
+#pragma unroll
+        for (int n = 0; n < 8; ++n) {
+          uint32_t bh0, bl0, bh1, bl1;
+          split_tf32(Ks[(n * 8 + g) * kKs + ks * 8 + t], bh0, bl0);
+          split_tf32(Ks[(n * 8 + g) * kKs + ks * 8 + t + 4], bh1, bl1);
+          mma_3xtf32(sacc[0][n], qh[0][ks], ql[0][ks], bh0, bh1, bl0, bl1);
+          mma_3xtf32(sacc[1][n], qh[1][ks], ql[1][ks], bh0, bh1, bl0, bl1);
+        }
+      // softmax step on the fragments: accumulator e -> row (e >> 1) * 8 + g of the tile, column 2t + (e & 1)
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf) {
+          float mx = -INFINITY;
+#pragma unroll
+          for (int n = 0; n < 8; ++n)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+              const float sv = fl[n * 8 + 2 * t + e] ? sacc[mt][n][hf * 2 + e] * scale : -INFINITY;   // key mask
+              sacc[mt][n][hf * 2 + e] = sv;
+              mx = fmaxf(mx, sv);
+            }
+          mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
+          mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
+          const float m_new = fmaxf(m_run[mt][hf], mx);
+          const float m_use = m_new == -INFINITY ? 0.f : m_new;   // no valid key yet: every p and alpha below is 0
+          const float alpha = expf(m_run[mt][hf] - m_use);
+          float sum = 0.f;
+#pragma unroll
+          for (int n = 0; n < 8; ++n)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+              const float pv = expf(sacc[mt][n][hf * 2 + e] - m_use);
+              sacc[mt][n][hf * 2 + e] = pv;
+              sum += pv;
+            }
+          sum += __shfl_xor_sync(0xffffffffu, sum, 1);
+          sum += __shfl_xor_sync(0xffffffffu, sum, 2);
+          m_run[mt][hf] = m_new;
+          l_run[mt][hf] = l_run[mt][hf] * alpha + sum;
+#pragma unroll
+          for (int n = 0; n < 4; ++n) {
+            oacc[mt][n][hf * 2] *= alpha;
+            oacc[mt][n][hf * 2 + 1] *= alpha;
+          }
+          float* prow = Ps + (mt * 16 + hf * 8 + g) * kCkPS + 2 * t;
+#pragma unroll
+          for (int n = 0; n < 8; ++n)
+            *reinterpret_cast<float2*>(prow + n * 8) = make_float2(sacc[mt][n][hf * 2], sacc[mt][n][hf * 2 + 1]);
+          const int row = l0 + mt * 16 + hf * 8 + g;
+          if (weights && row < L) {                     // one chunk (T <= 64): l is final, the probabilities are
+            const float inv = 1.f / l_run[mt][hf];
+            float* wrow = weights + ((static_cast<size_t>(b) * H + h) * L + row) * T;
+#pragma unroll
+            for (int n = 0; n < 8; ++n)
+#pragma unroll
+              for (int e = 0; e < 2; ++e) {
+                const int j = n * 8 + 2 * t + e;
+                if (j < T) wrow[j] = sacc[mt][n][hf * 2 + e] * inv;
+              }
+          }
+        }
+      __syncwarp();
+#pragma unroll
+      for (int kk = 0; kk < 8; ++kk) {
+        uint32_t ah[2][4], al[2][4];
+#pragma unroll
+        for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+          for (int e = 0; e < 4; ++e)
+            split_tf32(Ps[(mt * 16 + g + (e & 1) * 8) * kCkPS + kk * 8 + t + (e >> 1) * 4], ah[mt][e], al[mt][e]);
+#pragma unroll
+        for (int n = 0; n < 4; ++n) {
+          uint32_t bh0, bl0, bh1, bl1;
+          split_tf32(Vs[(kk * 8 + t) * kVs + n * 8 + g], bh0, bl0);
+          split_tf32(Vs[(kk * 8 + t + 4) * kVs + n * 8 + g], bh1, bl1);
+          mma_3xtf32(oacc[0][n], ah[0], al[0], bh0, bh1, bl0, bl1);
+          mma_3xtf32(oacc[1][n], ah[1], al[1], bh0, bh1, bl0, bl1);
+        }
+      }
+    }
+    __syncthreads();                                    // every warp is done with stage c & 1 (and its own P tile)
+  }
+  if (!active) return;
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int hf = 0; hf < 2; ++hf) {
+      const int row = l0 + mt * 16 + hf * 8 + g;
+      if (row < L) {
+        const float inv = 1.f / l_run[mt][hf];          // l = 0 (every key masked): NaN, like the reference
+        const size_t e0 = (static_cast<size_t>(b) * L + row) * (H * kHd) + h * kHd + 2 * t;
+#pragma unroll
+        for (int n = 0; n < 4; ++n)
+          attn_store2(out, e0 + n * 8, no_round, oacc[mt][n][hf * 2] * inv, oacc[mt][n][hf * 2 + 1] * inv);
+      }
+    }
+}
+
+static int launch_attn_chunked(const float* q, const float* k, const float* v, const int* mask, float* out, float* weights,
+                               int B, int H, int L, int T, int ld_q, int ld_kv, int no_round, int q_per_kv, cudaStream_t st) {
+  VQA_REQUIRE(q_per_kv >= 1 && B >= 1 && B % q_per_kv == 0, VQA_E_INVALID, "attn_chunked: the batch must be a multiple of q_per_kv");
+  VQA_REQUIRE(L >= 1 && L <= 512 && T >= 1 && T <= 512, VQA_E_INVALID, "attn_chunked: 1..512 queries and 1..512 keys");
+  VQA_REQUIRE(weights == nullptr || T <= kChunk, VQA_E_INVALID,
+              "attn_chunked: attention weights are stored for at most 64 keys (one chunk)");
+  const int qblocks = (L + 31) / 32;
+  const int ctas = (qblocks + kCkWarps - 1) / kCkWarps;   // per (pair, head)
+  const int warps = (qblocks + ctas - 1) / ctas;          // as few idle warps as the split allows
+  const size_t smem = static_cast<size_t>(kCkSmemFloats - (kCkWarps - warps) * 32 * kCkPS) * sizeof(float);
+  static bool attr_set[kMaxDevices] = {};
+  int dev = 0;
+  VQA_CUDA_OK(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= kMaxDevices || !attr_set[dev]) {
+    VQA_CUDA_OK(cudaFuncSetAttribute(reinterpret_cast<const void*>(&attn_chunked_kernel),
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, kCkSmemFloats * static_cast<int>(sizeof(float))));
+    if (dev >= 0 && dev < kMaxDevices) attr_set[dev] = true;
+  }
+  VQA_CUDA_OK(vqa_launch(attn_chunked_kernel, dim3(B * H, ctas), dim3(warps * 32), smem, st, q, k, v, mask, out, weights, H,
+                         L, T, ld_q, ld_kv, no_round, q_per_kv));
+  VQA_LAUNCH_OK("attn_chunked_kernel");
   return VQA_OK;
 }
 
@@ -1789,6 +2019,19 @@ int run_misc_op(const VqaOp& op, const uint64_t* ext, int n_ext, cudaStream_t st
                          PTR(float*, CROSS_ATTN_P_out), PTR(float*, CROSS_ATTN_P_weights), B, H, L, T, I[CROSS_ATTN_I_ld_q],
                          I[CROSS_ATTN_I_ld_kv], I[CROSS_ATTN_I_no_round], I[CROSS_ATTN_I_q_per_kv] > 0 ? I[CROSS_ATTN_I_q_per_kv] : 1, st);
     }
+    case VQA_OP_ATTN_CHUNKED: {
+      const int L = I[ATTN_CHUNKED_I_L], T = I[ATTN_CHUNKED_I_T], H = I[ATTN_CHUNKED_I_H], B = I[ATTN_CHUNKED_I_B];
+      VQA_REQUIRE(I[ATTN_CHUNKED_I_hd] == kHd && H >= 1, VQA_E_INVALID, "attn_chunked: head_dim=32");
+      const float* kv = PTR(const float*, ATTN_CHUNKED_P_kv);
+      VQA_REQUIRE(I[ATTN_CHUNKED_I_ld_q] % 4 == 0 && I[ATTN_CHUNKED_I_ld_kv] % 4 == 0 && I[ATTN_CHUNKED_I_k_off] % 4 == 0 &&
+                      I[ATTN_CHUNKED_I_v_off] % 4 == 0 && (reinterpret_cast<uintptr_t>(kv) & 15) == 0 &&
+                      (reinterpret_cast<uintptr_t>(PTR(float*, ATTN_CHUNKED_P_out)) & 15) == 0,
+                  VQA_E_ALIGN, "attn_chunked: K / V and the output must be 16-byte aligned, leading dimensions multiples of 4");
+      return launch_attn_chunked(PTR(const float*, ATTN_CHUNKED_P_q), kv + I[ATTN_CHUNKED_I_k_off], kv + I[ATTN_CHUNKED_I_v_off],
+                                 PTR(const int*, ATTN_CHUNKED_P_mask), PTR(float*, ATTN_CHUNKED_P_out),
+                                 PTR(float*, ATTN_CHUNKED_P_weights), B, H, L, T, I[ATTN_CHUNKED_I_ld_q], I[ATTN_CHUNKED_I_ld_kv],
+                                 I[ATTN_CHUNKED_I_no_round], I[ATTN_CHUNKED_I_q_per_kv], st);
+    }
     case VQA_OP_POOL_GATE_LN: {
       const int phase = I[POOL_GATE_LN_I_phase];
       VQA_REQUIRE(I[POOL_GATE_LN_I_D] == 256, VQA_E_INVALID, "pool_gate_ln: D must be 256");
@@ -1840,6 +2083,7 @@ const char* misc_kernel_name(int kind) {
     case VQA_OP_LAYERNORM: return "layernorm256_kernel";
     case VQA_OP_SELF_ATTN: return "attn_mma_kernel(self)";
     case VQA_OP_CROSS_ATTN: return "attn_mma_kernel(cross)";
+    case VQA_OP_ATTN_CHUNKED: return "attn_chunked_kernel";
     case VQA_OP_POOL_GATE_LN: return "pool_gate_ln_kernel";
     case VQA_OP_SOFTMAX_TOPK: return "softmax_topk_kernel";
     default: return "?";

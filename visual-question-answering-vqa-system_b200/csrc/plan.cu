@@ -49,6 +49,7 @@ const FieldCount kFields[VQA_OP_KIND_MAX] = {
     {SPLIT_TF32_NI, SPLIT_TF32_NP, SPLIT_TF32_NF},
     {STEM_POOL_NI, STEM_POOL_NP, STEM_POOL_NF},
     {MLP_CHAIN_NI, MLP_CHAIN_NP, MLP_CHAIN_NF},
+    {ATTN_CHUNKED_NI, ATTN_CHUNKED_NP, ATTN_CHUNKED_NF},
 };
 static_assert(MLP_CHAIN_NP <= VQA_OP_NP, "VqaOp.p too small for the chain op");
 static_assert(GEMM_NI <= VQA_OP_NI, "VqaOp.i too small for the gemm op");

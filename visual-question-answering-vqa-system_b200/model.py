@@ -20,7 +20,7 @@ import torch.nn.functional as F
 from .modules import AnswerHead, CustomResNet, MultimodalFusion, TransformerTextEncoder
 
 _SUPPORTED = ("The sm_100a engine is specialised for embed_dim=256, 8 heads, ffn_hidden_dim=1024 "
-              "(the reference defaults); layer counts, vocab/answer sizes, max_question_length<=64 "
+              "(the reference defaults); layer counts, vocab/answer sizes, max_question_length<=512 "
               "and the SE/spatial/gating ablation switches are free.")
 
 
@@ -63,7 +63,7 @@ class VQAModel(nn.Module):
         c = self.config
         if c["embed_dim"] != 256 or c["num_attention_heads"] != 8 or c["ffn_hidden_dim"] != 1024:
             raise NotImplementedError(_SUPPORTED)
-        if c["max_question_length"] > 64:
+        if c["max_question_length"] > 512:
             raise NotImplementedError(_SUPPORTED)
 
     def engine(self):

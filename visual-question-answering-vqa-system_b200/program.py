@@ -36,7 +36,7 @@ KINDS = {
     "ingest": 1, "gemm": 2, "maxpool": 3, "se_squeeze": 4, "se_excite": 5, "spatial_map": 6,
     "scale_relayout": 7, "embed": 8, "layernorm": 9, "self_attn": 10, "cross_attn": 11,
     "pool_gate_ln": 12, "softmax_topk": 13, "mask_prep": 14, "grid_to_nchw": 15,
-    "copy_rows": 16, "stage_tail": 17, "split_tf32": 18, "stem_pool": 19, "mlp_chain": 20,
+    "copy_rows": 16, "stage_tail": 17, "split_tf32": 18, "stem_pool": 19, "mlp_chain": 20, "attn_chunked": 21,
 }
 
 _GROUPS = [f"g_{k}{g}" for k in ("map", "delta", "acol", "chunks", "ntaps", "kbase", "tap0")
@@ -82,6 +82,8 @@ FIELDS: Dict[str, Dict[str, List[str]]] = {
     "mlp_chain": {"i": ["T", "D", "F", "Nn", "Nn_pad", "max_ctas", "CS"],
                   "p": ["ctx", "xres", "xout", "wo", "w1", "b1", "w2", "b2", "ln_g", "ln_b", "n_g", "n_b", "wn", "y"],
                   "f": ["eps", "eps_n"]},
+    "attn_chunked": {"i": ["B", "L", "H", "hd", "T", "ld_q", "ld_kv", "k_off", "v_off", "no_round", "q_per_kv"],
+                     "p": ["q", "kv", "mask", "out", "weights"], "f": []},
 }
 
 DT_BF16, DT_TF32, DT_F16 = 0, 1, 2      # gemm operand dtype
@@ -91,6 +93,11 @@ MASK_NONE, MASK_I64, MASK_F32, MASK_I32, MASK_U8 = 0, 1, 2, 3, 4
 # external slots (order of the ext[] array given to vqa_plan_run)
 EXT = {"images": 0, "ids": 1, "mask": 2, "logits": 3, "top_idx": 4, "top_probs": 5}
 MAX_CACHED_LAYERS = 8
+# attn_mma_kernel (self_attn / cross_attn) holds every key of a (pair, head) in one warp: up to 64.  Longer questions run
+# attn_chunked_kernel, which streams the keys in chunks of 64 (up to 512).  Programs of at most 64 tokens keep the
+# single-warp kernel, so their results stay bit for bit what they were (DESIGN.md, "Long questions").
+ATTN_MMA_MAX_L = 64
+MAX_QUESTION_LENGTH = 512
 TOPK_FUSED_MAX = 8   # kTopKMax in csrc/gemm_tcgen05.cu: winners an epilogue thread keeps; larger k uses softmax_topk_kernel
 # K/V of a cached image side (question-side programs): one slot per cross-attention layer
 EXT.update({f"kv{l}": 6 + l for l in range(MAX_CACHED_LAYERS)})
@@ -1042,8 +1049,13 @@ class Program(OpList):
                 if not (fuse_embed and layer == 0):
                     self.layernorm(p + ".ln1", xt, p + ".ln1.g", p + ".ln1.b", xn, T, rnd=True)
                 self.linear(p + ".qkv", xn, T, D, p + ".qkv.w", None, qkv, 3 * D)
-            self._op("self_attn", p + ".attn", dict(B=B, L=L, H=H, hd=D // H, ld_qkv=3 * D, no_round=self.out_mode),
-                     dict(qkv=qkv, mask=mask, out=ctx))
+            if L <= ATTN_MMA_MAX_L:
+                self._op("self_attn", p + ".attn", dict(B=B, L=L, H=H, hd=D // H, ld_qkv=3 * D, no_round=self.out_mode),
+                         dict(qkv=qkv, mask=mask, out=ctx))
+            else:
+                self._op("attn_chunked", p + ".attn", dict(B=B, L=L, H=H, hd=D // H, T=L, ld_q=3 * D, ld_kv=3 * D, k_off=D,
+                                                           v_off=2 * D, no_round=self.out_mode, q_per_kv=1),
+                         dict(q=qkv, kv=qkv, mask=mask, out=ctx))
             if chain:
                 q1 = f"text.{layer + 1}"
                 nxt = (q1 + ".ln1", q1 + ".qkv.w.h", qkv, 3 * D) if (q1 + ".qkv.w") in W else None
@@ -1110,9 +1122,12 @@ class Program(OpList):
             if self.want_aux:
                 wts = self._buf(f"aux.xattn.{layer}", f32, B, H, L, S * S)
                 self.xattn_weights.append(f"aux.xattn.{layer}")
-            self._op("cross_attn", p + ".attn", dict(B=B, L=L, H=H, hd=D // H, T=S * S, ld_q=D, ld_kv=2 * D, k_off=0, v_off=D,
-                                                     no_round=self.out_mode, q_per_kv=B // Bi),
-                     dict(q=qp, kv=kvs[layer], out=cx, weights=wts))
+            xi = dict(B=B, L=L, H=H, hd=D // H, T=S * S, ld_q=D, ld_kv=2 * D, k_off=0, v_off=D, no_round=self.out_mode,
+                      q_per_kv=B // Bi)
+            if L <= ATTN_MMA_MAX_L:
+                self._op("cross_attn", p + ".attn", xi, dict(q=qp, kv=kvs[layer], out=cx, weights=wts))
+            else:
+                self._op("attn_chunked", p + ".attn", xi, dict(q=qp, kv=kvs[layer], mask=None, out=cx, weights=wts))
             if not cached:
                 self.ops[-1].lane |= LANE_JOIN    # needs the side lane's q (layer 0) / K,V (layers >= 1)
             if layer == 0 and n_layers > 1 and not cached:   # side lane: K/V of every later layer, concurrent with this layer's chain

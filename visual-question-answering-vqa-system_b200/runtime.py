@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libvqa_b200.so")
 
 OP_NI, OP_NP, OP_NF = 160, 16, 4
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 
 class VqaOp(C.Structure):
