@@ -1163,12 +1163,145 @@ __global__ void embed_ln_kernel(const long long* __restrict__ ids, const float* 
   ln256_store(ln_dst, tok, lane, rnd, y);
 }
 
-constexpr int kHd = 32;
+// LayerNorm over the other embedding widths (D = 128 .. 512 in steps of 64), one warp per row as layernorm256_kernel:
+// a lane holds D / 32 values, loaded as D / 128 float4 (D % 128 == 0) or D / 64 float2 (D = 192, 320, 448) at vector
+// index lane + 32 j.  Statistics as ln256_apply: lane partial sums in register order, warp_sum, biased variance, eps
+// inside the sqrt; the mean and the variance divide by D (at 256 that is ln256_apply's exact multiplication by 1 / 256).
+// layernorm256_kernel stays the kernel of D = 256.
+template <int D>
+struct LnRow {
+  static constexpr int VW = D % 128 == 0 ? 4 : 2;      // floats per vector load
+  static constexpr int NP = D / (32 * VW);              // vector loads per lane
+  static constexpr int NV = D / 32;                     // values per lane
+  static_assert(D % 64 == 0 && D >= 128 && D <= 512, "LayerNorm widths: 128 .. 512 in steps of 64");
+};
+template <int D, bool kLdg>
+__device__ __forceinline__ void ln_load(const float* row, int lane, float (&x)[LnRow<D>::NV]) {
+#pragma unroll
+  for (int p = 0; p < LnRow<D>::NP; ++p) {
+    if constexpr (LnRow<D>::VW == 4) {
+      const float4* r4 = reinterpret_cast<const float4*>(row) + lane + 32 * p;
+      const float4 a = kLdg ? __ldg(r4) : *r4;
+      x[4 * p] = a.x; x[4 * p + 1] = a.y; x[4 * p + 2] = a.z; x[4 * p + 3] = a.w;
+    } else {
+      const float2* r2 = reinterpret_cast<const float2*>(row) + lane + 32 * p;
+      const float2 a = kLdg ? __ldg(r2) : *r2;
+      x[2 * p] = a.x; x[2 * p + 1] = a.y;
+    }
+  }
+}
+template <int D>
+__device__ __forceinline__ void ln_apply(const float (&x)[LnRow<D>::NV], const float (&g)[LnRow<D>::NV],
+                                         const float (&bb)[LnRow<D>::NV], float eps, float (&y)[LnRow<D>::NV]) {
+  constexpr int NV = LnRow<D>::NV;
+  float s = 0.f;
+#pragma unroll
+  for (int k = 0; k < NV; ++k) s += x[k];
+  const float mean = warp_sum(s) / static_cast<float>(D);
+  float v[NV], q = 0.f;
+#pragma unroll
+  for (int k = 0; k < NV; ++k) { v[k] = x[k] - mean; q += v[k] * v[k]; }
+  const float rstd = rsqrtf(warp_sum(q) / static_cast<float>(D) + eps);
+#pragma unroll
+  for (int k = 0; k < NV; ++k) y[k] = v[k] * rstd * g[k] + bb[k];
+}
+// Store a row: rnd 0 = fp32, 1 = tf32-rounded fp32, 2 = fp16 (operand of an fp16 Linear).
+template <int D>
+__device__ __forceinline__ void ln_store(float* dst, int row, int lane, int rnd, const float (&y)[LnRow<D>::NV]) {
+  constexpr int VW = LnRow<D>::VW, NP = LnRow<D>::NP;
+  if (rnd == 2) {
+    __half* h = reinterpret_cast<__half*>(dst) + static_cast<size_t>(row) * D;
+#pragma unroll
+    for (int p = 0; p < NP; ++p) {
+      if constexpr (VW == 4)
+        reinterpret_cast<uint2*>(h)[lane + 32 * p] = make_uint2(pack_f16x2(y[4 * p], y[4 * p + 1]), pack_f16x2(y[4 * p + 2], y[4 * p + 3]));
+      else
+        reinterpret_cast<uint32_t*>(h)[lane + 32 * p] = pack_f16x2(y[2 * p], y[2 * p + 1]);
+    }
+    return;
+  }
+  float* o = dst + static_cast<size_t>(row) * D;
+#pragma unroll
+  for (int p = 0; p < NP; ++p) {
+    float r[VW];
+#pragma unroll
+    for (int e = 0; e < VW; ++e) r[e] = rnd ? round_tf32_rna(y[VW * p + e]) : y[VW * p + e];
+    if constexpr (VW == 4)
+      reinterpret_cast<float4*>(o)[lane + 32 * p] = make_float4(r[0], r[1], r[2], r[3]);
+    else
+      reinterpret_cast<float2*>(o)[lane + 32 * p] = make_float2(r[0], r[1]);
+  }
+}
+
+template <int D>
+__global__ void layernorm_kernel(const float* __restrict__ src, const float* __restrict__ gamma,
+                                 const float* __restrict__ beta, float* __restrict__ dst,
+                                 const float* __restrict__ pos, int rows, int ld, int mode, int rnd, int S, int Pg,
+                                 int RPIg, float eps, const LnExtra ex) {
+  constexpr int NV = LnRow<D>::NV;
+  pdl_launch_dependents();
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  float g[NV], bb[NV];                                   // weights: fetched before waiting for the producer of the rows
+  ln_load<D, true>(gamma, lane, g);
+  ln_load<D, true>(beta, lane, bb);
+  pdl_wait();
+  if (row >= rows) return;
+  size_t srow = row;
+  int pix = 0;
+  if (mode == 1) {
+    const int n = row / (S * S);
+    pix = row - n * S * S;
+    srow = static_cast<size_t>(n) * RPIg + (pix / S) * Pg + (pix % S);
+  }
+  float x[NV], y[NV];
+  ln_load<D, false>(src + srow * ld, lane, x);
+  ln_apply<D>(x, g, bb, eps, y);
+  if (mode == 1 && pos) {
+    float p[NV];
+    ln_load<D, false>(pos + static_cast<size_t>(pix) * D, lane, p);
+#pragma unroll
+    for (int k = 0; k < NV; ++k) y[k] += p[k];
+  }
+  if (ex.gamma2 != nullptr) {
+    float g2[NV], b2[NV], z[NV];
+    ln_load<D, true>(ex.gamma2, lane, g2);
+    ln_load<D, true>(ex.beta2, lane, b2);
+    ln_apply<D>(y, g2, b2, eps, z);
+    ln_store<D>(ex.dst2, row, lane, ex.rnd2, z);
+  }
+  if (ex.gamma3 != nullptr) {
+    float g3[NV], b3[NV], z[NV];
+    ln_load<D, true>(ex.gamma3, lane, g3);
+    ln_load<D, true>(ex.beta3, lane, b3);
+    ln_apply<D>(y, g3, b3, eps, z);
+    ln_store<D>(ex.dst3, row, lane, ex.rnd3, z);
+  }
+  ln_store<D>(dst, row, lane, rnd, y);
+}
+
+typedef void (*LayerNormFn)(const float*, const float*, const float*, float*, const float*, int, int, int, int, int, int, int,
+                            float, const LnExtra);
+
+// The LayerNorm of width D: layernorm256_kernel at 256, layernorm_kernel<D> at the other widths; nullptr outside them.
+static LayerNormFn layernorm_fn(int D) {
+  switch (D) {
+    case 128: return &layernorm_kernel<128>;
+    case 192: return &layernorm_kernel<192>;
+    case 256: return &layernorm256_kernel;
+    case 320: return &layernorm_kernel<320>;
+    case 384: return &layernorm_kernel<384>;
+    case 448: return &layernorm_kernel<448>;
+    case 512: return &layernorm_kernel<512>;
+    default: return nullptr;
+  }
+}
+
 constexpr int kAttnWarps = 4;
 
 // ------------------------------------------------------------------------------------------------
-// Attention core, one WARP per (pair, head): softmax(Q K^T / sqrt(32) [+ key mask]) V with head_dim 32, up
-// to 64 queries (blocks of 32) and up to 64 keys.  Self-attention (models/text_encoder.py:229-259; keys
+// Attention core, one WARP per (pair, head): softmax(Q K^T / sqrt(HD) [+ key mask]) V with head_dim HD = 16, 32 or 64,
+// up to 64 queries (blocks of 32) and up to 64 keys.  Self-attention (models/text_encoder.py:229-259; keys
 // with mask == 0 get -inf, a fully masked row yields NaN exactly like the reference, SURVEY T5) and
 // cross-attention over the 49 image tokens (models/cross_attention.py:164-197, no mask) share it.
 // S = Q K^T and O = P V run on mma.sync m16n8k8 with the 3xTF32 split (x = hi + lo; lo*hi + hi*lo + hi*hi:
@@ -1205,13 +1338,62 @@ __device__ __forceinline__ void attn_store2(float* out, size_t e, int no_round, 
   }
 }
 
-constexpr int kKs = 36, kVs = 40;                       // padded row strides (floats): conflict-free fragment loads
-__host__ __device__ constexpr int attn_mma_kreg(int nt) {           // K rows, later the probability tile [32][nt*8+4]
-  return nt * 8 * kKs > 32 * (nt * 8 + 4) ? nt * 8 * kKs : 32 * (nt * 8 + 4);
+// Head widths: HD = 16, 32 or 64 (head_dim = embed_dim / num_heads).  Padded shared-memory row strides HD + 4 (K) and
+// HD + 8 (V) keep the fragment loads conflict-free at every width (g * stride + t, resp. t * stride + g, cover 32 banks).
+__host__ __device__ constexpr int attn_ks(int hd) { return hd + 4; }
+__host__ __device__ constexpr int attn_vs(int hd) { return hd + 8; }
+__host__ __device__ constexpr int attn_mma_kreg(int nt, int hd) {   // K rows, later the probability tile [32][nt*8+4]
+  return nt * 8 * attn_ks(hd) > 32 * (nt * 8 + 4) ? nt * 8 * attn_ks(hd) : 32 * (nt * 8 + 4);
 }
-__host__ __device__ constexpr int attn_mma_warp_floats(int nt) { return attn_mma_kreg(nt) + nt * 8 * kVs; }
+__host__ __device__ constexpr int attn_mma_warp_floats(int nt, int hd) { return attn_mma_kreg(nt, hd) + nt * 8 * attn_vs(hd); }
+// The reference divides the scores by sqrt(head_dim) (CrossAttention / MultiHeadSelfAttention).  1 / sqrt(16) and
+// 1 / sqrt(64) are powers of two, so multiplying by them is that division exactly; head_dim 32 keeps rsqrtf(32).
+template <int HD>
+__device__ __forceinline__ float attn_scale() {
+  static_assert(HD == 16 || HD == 32 || HD == 64, "head_dim 16, 32 or 64");
+  if constexpr (HD == 32) return rsqrtf(static_cast<float>(HD));
+  else return HD == 16 ? 0.25f : 0.125f;
+}
+// Q fragments of one 8-wide k step (rows g, g+8 of each 16-row tile; dims t, t+4), split into tf32 hi / lo.  Up to
+// head_dim 32 a warp keeps every k step's fragments in registers; at 64 they would take 128 registers next to the 64 of
+// the score and the 64 of the context accumulators, so they are reloaded (from L1) for every k step instead.
+template <int HD>
+struct QFrags {
+  static constexpr bool kRegs = HD <= 32;
+  uint32_t h[2][kRegs ? HD / 8 : 1][4], l[2][kRegs ? HD / 8 : 1][4];
+  __device__ __forceinline__ void load(const float* qb, int ld_q, int L, int l0, int g, int t) {
+    if constexpr (kRegs) {
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int ks = 0; ks < HD / 8; ++ks)
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const int row = l0 + mt * 16 + g + (e & 1) * 8, col = ks * 8 + t + (e >> 1) * 4;
+            const float x = row < L ? __ldg(qb + static_cast<size_t>(row) * ld_q + col) : 0.f;
+            split_tf32(x, h[mt][ks][e], l[mt][ks][e]);
+          }
+    }
+  }
+  __device__ __forceinline__ void step(const float* qb, int ld_q, int L, int l0, int g, int t, int ks, uint32_t (&fh)[2][4],
+                                       uint32_t (&fl)[2][4]) const {
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        if constexpr (kRegs) {
+          fh[mt][e] = h[mt][ks][e];
+          fl[mt][e] = l[mt][ks][e];
+        } else {
+          const int row = l0 + mt * 16 + g + (e & 1) * 8, col = ks * 8 + t + (e >> 1) * 4;
+          const float x = row < L ? __ldg(qb + static_cast<size_t>(row) * ld_q + col) : 0.f;
+          split_tf32(x, fh[mt][e], fl[mt][e]);
+        }
+      }
+  }
+};
 
-template <int NT>
+template <int NT, int HD>
 __global__ void __launch_bounds__(kAttnWarps * 32)
 attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v,
                 const int* __restrict__ mask, float* __restrict__ out, float* __restrict__ weights, int n_units,
@@ -1219,25 +1401,26 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
   pdl_launch_dependents();
   pdl_wait();
   extern __shared__ __align__(16) float sm[];
+  constexpr int kKs = attn_ks(HD), kVs = attn_vs(HD);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = lane >> 2, t = lane & 3;
   const int unit = blockIdx.x * kAttnWarps + warp;     // (pair, head)
   if (unit >= n_units) return;
   const int b = unit / H, h = unit - b * H;
   constexpr int PS = NT * 8 + 4;                        // probability tile row stride
-  float* Ks = sm + warp * attn_mma_warp_floats(NT);
+  float* Ks = sm + warp * attn_mma_warp_floats(NT, HD);
   float* Ps = Ks;
-  float* Vs = Ks + attn_mma_kreg(NT);
-  const float* qb = q + static_cast<size_t>(b) * L * ld_q + h * kHd;
+  float* Vs = Ks + attn_mma_kreg(NT, HD);
+  const float* qb = q + static_cast<size_t>(b) * L * ld_q + h * HD;
   const int bkv = b / q_per_kv;                         // q_per_kv consecutive queries share one image's K / V
-  const float* kb = k + static_cast<size_t>(bkv) * T * ld_kv + h * kHd;
-  const float* vb = v + static_cast<size_t>(bkv) * T * ld_kv + h * kHd;
+  const float* kb = k + static_cast<size_t>(bkv) * T * ld_kv + h * HD;
+  const float* vb = v + static_cast<size_t>(bkv) * T * ld_kv + h * HD;
   // K / V rows go global -> shared with cp.async (all 16-byte pieces of the head in flight at once; rows beyond T
   // are zero-filled through the src-size operand).  A register-staged loop serialised 14 + 14 DRAM/L2 round trips
   // per warp and was 1/3 of the kernel's stall samples (ncu source view, profiles/r01_h_*).
   auto stage_rows = [&](float* dst, int stride, const float* src) {
-    for (int i = lane; i < NT * 8 * 8; i += 32) {
-      const int r = i >> 3, c4 = i & 7;
+    for (int i = lane; i < NT * 8 * (HD / 4); i += 32) {
+      const int r = i / (HD / 4), c4 = i % (HD / 4);
       const float* g = src + static_cast<size_t>(r < T ? r : 0) * ld_kv + c4 * 4;
       const uint32_t d = static_cast<uint32_t>(__cvta_generic_to_shared(dst + r * stride + c4 * 4));
       asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d), "l"(g), "r"(r < T ? 16 : 0) : "memory");
@@ -1252,23 +1435,13 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
       const int j = n * 8 + 2 * t + e;
       mb[n][e] = (j < T && (mask == nullptr || mask[b * T + j] != 0)) ? 0.f : -INFINITY;   // self-attention only (q_per_kv = 1)
     }
-  const float scale = rsqrtf(static_cast<float>(kHd));
+  const float scale = attn_scale<HD>();
   for (int l0 = 0; l0 < L; l0 += 32) {
     __syncwarp();
     stage_rows(Ks, kKs, kb);                            // K rows (the region is reused for P below)
     asm volatile("cp.async.commit_group;" ::: "memory");
-    // Q fragments (rows g, g+8 of each 16-row tile; dims t, t+4 of each 8-wide k step), pre-split
-    uint32_t qh[2][4][4], ql[2][4][4];
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks)
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const int row = l0 + mt * 16 + g + (e & 1) * 8, col = ks * 8 + t + (e >> 1) * 4;
-          const float x = row < L ? __ldg(qb + static_cast<size_t>(row) * ld_q + col) : 0.f;
-          split_tf32(x, qh[mt][ks][e], ql[mt][ks][e]);
-        }
+    QFrags<HD> qf;                                      // Q fragments, pre-split (head_dim <= 32)
+    qf.load(qb, ld_q, L, l0, g, t);
     asm volatile("cp.async.wait_group 0;" ::: "memory");   // this lane's K (and, first pass, V) pieces have landed
     __syncwarp();
     float sacc[2][NT][4];
@@ -1279,15 +1452,18 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
 #pragma unroll
         for (int e = 0; e < 4; ++e) sacc[mt][n][e] = 0.f;
 #pragma unroll
-    for (int ks = 0; ks < 4; ++ks)
+    for (int ks = 0; ks < HD / 8; ++ks) {
+      uint32_t fh[2][4], fl[2][4];
+      qf.step(qb, ld_q, L, l0, g, t, ks, fh, fl);
 #pragma unroll
       for (int n = 0; n < NT; ++n) {
         uint32_t bh0, bl0, bh1, bl1;
         split_tf32(Ks[(n * 8 + g) * kKs + ks * 8 + t], bh0, bl0);
         split_tf32(Ks[(n * 8 + g) * kKs + ks * 8 + t + 4], bh1, bl1);
-        mma_3xtf32(sacc[0][n], qh[0][ks], ql[0][ks], bh0, bh1, bl0, bl1);
-        mma_3xtf32(sacc[1][n], qh[1][ks], ql[1][ks], bh0, bh1, bl0, bl1);
+        mma_3xtf32(sacc[0][n], fh[0], fl[0], bh0, bh1, bl0, bl1);
+        mma_3xtf32(sacc[1][n], fh[1], fl[1], bh0, bh1, bl0, bl1);
       }
+    }
     __syncwarp();                                       // every lane is done with K: the region becomes P
     // softmax on the fragments: accumulator e -> row (e >> 1) * 8 + g of the tile, column 2t + (e & 1)
 #pragma unroll
@@ -1328,11 +1504,11 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
       float* wb = weights + ((static_cast<size_t>(b) * H + h) * L + l0) * T;
       for (int i = lane; i < rows * T; i += 32) wb[i] = Ps[(i / T) * PS + (i % T)];
     }
-    float oacc[2][4][4];
+    float oacc[2][HD / 8][4];
 #pragma unroll
     for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
-      for (int n = 0; n < 4; ++n)
+      for (int n = 0; n < HD / 8; ++n)
 #pragma unroll
         for (int e = 0; e < 4; ++e) oacc[mt][n][e] = 0.f;
 #pragma unroll
@@ -1344,7 +1520,7 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
         for (int e = 0; e < 4; ++e)
           split_tf32(Ps[(mt * 16 + g + (e & 1) * 8) * PS + kk * 8 + t + (e >> 1) * 4], ah[mt][e], al[mt][e]);
 #pragma unroll
-      for (int n = 0; n < 4; ++n) {
+      for (int n = 0; n < HD / 8; ++n) {
         uint32_t bh0, bl0, bh1, bl1;
         split_tf32(Vs[(kk * 8 + t) * kVs + n * 8 + g], bh0, bl0);
         split_tf32(Vs[(kk * 8 + t + 4) * kVs + n * 8 + g], bh1, bl1);
@@ -1358,9 +1534,9 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
       for (int hf = 0; hf < 2; ++hf) {
         const int row = l0 + mt * 16 + hf * 8 + g;
         if (row < L) {
-          const size_t e0 = (static_cast<size_t>(b) * L + row) * (H * kHd) + h * kHd + 2 * t;
+          const size_t e0 = (static_cast<size_t>(b) * L + row) * (H * HD) + h * HD + 2 * t;
 #pragma unroll
-          for (int n = 0; n < 4; ++n) attn_store2(out, e0 + n * 8, no_round, oacc[mt][n][hf * 2], oacc[mt][n][hf * 2 + 1]);
+          for (int n = 0; n < HD / 8; ++n) attn_store2(out, e0 + n * 8, no_round, oacc[mt][n][hf * 2], oacc[mt][n][hf * 2 + 1]);
         }
       }
   }
@@ -1369,23 +1545,34 @@ attn_mma_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
 typedef void (*AttnFn)(const float*, const float*, const float*, const int*, float*, float*, int, int, int, int, int, int, int,
                        int);
 
+// head_dim -> index of its instantiations (16, 32, 64 -> 0, 1, 2), -1 for any other width
+static int attn_hd_index(int hd) { return hd == 16 ? 0 : hd == 32 ? 1 : hd == 64 ? 2 : -1; }
+
+template <int HD>
+static AttnFn attn_mma_fn(int ntt) {
+  return ntt == 3 ? static_cast<AttnFn>(&attn_mma_kernel<3, HD>) : ntt == 4 ? static_cast<AttnFn>(&attn_mma_kernel<4, HD>)
+       : ntt == 7 ? static_cast<AttnFn>(&attn_mma_kernel<7, HD>) : static_cast<AttnFn>(&attn_mma_kernel<8, HD>);
+}
+
 static int launch_attn(const float* q, const float* k, const float* v, const int* mask, float* out, float* weights, int B,
-                       int H, int L, int T, int ld_q, int ld_kv, int no_round, int q_per_kv, cudaStream_t st) {
+                       int H, int L, int T, int hd, int ld_q, int ld_kv, int no_round, int q_per_kv, cudaStream_t st) {
   VQA_REQUIRE(q_per_kv >= 1 && B % q_per_kv == 0, VQA_E_INVALID, "attention: the batch must be a multiple of q_per_kv");
+  const int hdi = attn_hd_index(hd);
+  VQA_REQUIRE(hdi >= 0, VQA_E_INVALID, "attention: head_dim must be 16, 32 or 64");
   const int nt = (T + 7) / 8;
   VQA_REQUIRE(nt >= 1 && nt <= 8, VQA_E_INVALID, "attention: 1..64 keys");
   const int ntt = nt <= 3 ? 3 : nt <= 4 ? 4 : nt <= 7 ? 7 : 8;
-  AttnFn fn = ntt == 3 ? static_cast<AttnFn>(&attn_mma_kernel<3>) : ntt == 4 ? static_cast<AttnFn>(&attn_mma_kernel<4>)
-            : ntt == 7 ? static_cast<AttnFn>(&attn_mma_kernel<7>) : static_cast<AttnFn>(&attn_mma_kernel<8>);
-  const size_t smem = static_cast<size_t>(kAttnWarps) * attn_mma_warp_floats(ntt) * sizeof(float);
+  AttnFn fn = hd == 16 ? attn_mma_fn<16>(ntt) : hd == 32 ? attn_mma_fn<32>(ntt) : attn_mma_fn<64>(ntt);
+  // head_dim 64, 64 keys: 35 KB per warp, 140 KB per CTA (one CTA per SM)
+  const size_t smem = static_cast<size_t>(kAttnWarps) * attn_mma_warp_floats(ntt, hd) * sizeof(float);
   // cudaFuncSetAttribute is per device (context): remember it per (device, instantiation)
-  static bool attr_set[kMaxDevices][9] = {};
+  static bool attr_set[kMaxDevices][3][9] = {};
   int dev = 0;
   VQA_CUDA_OK(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= kMaxDevices || !attr_set[dev][ntt]) {
+  if (dev < 0 || dev >= kMaxDevices || !attr_set[dev][hdi][ntt]) {
     VQA_CUDA_OK(cudaFuncSetAttribute(reinterpret_cast<const void*>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      static_cast<int>(smem)));
-    if (dev >= 0 && dev < kMaxDevices) attr_set[dev][ntt] = true;
+    if (dev >= 0 && dev < kMaxDevices) attr_set[dev][hdi][ntt] = true;
   }
   VQA_CUDA_OK(vqa_launch(fn, dim3((B * H + kAttnWarps - 1) / kAttnWarps), dim3(kAttnWarps * 32), smem, st, q, k, v, mask, out,
                          weights, B * H, H, L, T, ld_q, ld_kv, no_round, q_per_kv));
@@ -1407,10 +1594,12 @@ static int launch_attn(const float* q, const float* k, const float* v, const int
 // element, as in the reference (SURVEY T5).
 constexpr int kChunk = 64;                               // keys per chunk (8 tiles of 8)
 constexpr int kCkWarps = 4;
-constexpr int kCkStage = kChunk * (kKs + kVs);           // floats of one K + V chunk
+__host__ __device__ constexpr int ck_stage(int hd) { return kChunk * (attn_ks(hd) + attn_vs(hd)); }   // floats of one K + V chunk
 constexpr int kCkPS = kChunk + 4;                        // probability tile row stride
-constexpr int kCkSmemFloats = 2 * kCkStage + 2 * kChunk + kCkWarps * 32 * kCkPS;   // K/V x 2, key flags x 2, P per warp
+// K/V x 2, key flags x 2, P per warp: 58 / 74 / 107 KB at head_dim 16 / 32 / 64
+__host__ __device__ constexpr int ck_smem_floats(int hd) { return 2 * ck_stage(hd) + 2 * kChunk + kCkWarps * 32 * kCkPS; }
 
+template <int HD>
 __global__ void __launch_bounds__(kCkWarps * 32)
 attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v,
                     const int* __restrict__ mask, float* __restrict__ out, float* __restrict__ weights, int H, int L, int T,
@@ -1418,6 +1607,7 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
   pdl_launch_dependents();
   pdl_wait();
   extern __shared__ __align__(16) float sm[];
+  constexpr int kKs = attn_ks(HD), kVs = attn_vs(HD), kCkStage = ck_stage(HD);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int unit = blockIdx.x;                          // (pair, head)
@@ -1426,17 +1616,17 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
   const bool active = l0 < L;
   int* flags = reinterpret_cast<int*>(sm + 2 * kCkStage);   // [2][kChunk]: 1 = a valid key
   float* Ps = sm + 2 * kCkStage + 2 * kChunk + warp * 32 * kCkPS;
-  const float* qb = q + static_cast<size_t>(b) * L * ld_q + h * kHd;
+  const float* qb = q + static_cast<size_t>(b) * L * ld_q + h * HD;
   const int bkv = b / q_per_kv;                         // q_per_kv consecutive queries share one image's K / V
-  const float* kb = k + static_cast<size_t>(bkv) * T * ld_kv + h * kHd;
-  const float* vb = v + static_cast<size_t>(bkv) * T * ld_kv + h * kHd;
+  const float* kb = k + static_cast<size_t>(bkv) * T * ld_kv + h * HD;
+  const float* vb = v + static_cast<size_t>(bkv) * T * ld_kv + h * HD;
   const int n_chunks = (T + kChunk - 1) / kChunk;
   // chunk c -> stage c & 1: K and V rows (rows beyond T zero-filled through the src-size operand) and the key flags
   auto stage = [&](int c) {
     float* Ks = sm + (c & 1) * kCkStage;
     float* Vs = Ks + kChunk * kKs;
-    for (int i = threadIdx.x; i < kChunk * 8; i += blockDim.x) {
-      const int r = i >> 3, c4 = i & 7, j = c * kChunk + r;
+    for (int i = threadIdx.x; i < kChunk * (HD / 4); i += blockDim.x) {
+      const int r = i / (HD / 4), c4 = i % (HD / 4), j = c * kChunk + r;
       const size_t off = static_cast<size_t>(j < T ? j : 0) * ld_kv + c4 * 4;
       const uint32_t dk = static_cast<uint32_t>(__cvta_generic_to_shared(Ks + r * kKs + c4 * 4));
       const uint32_t dv = static_cast<uint32_t>(__cvta_generic_to_shared(Vs + r * kVs + c4 * 4));
@@ -1450,20 +1640,10 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
     asm volatile("cp.async.commit_group;" ::: "memory");
   };
   stage(0);
-  // Q fragments (rows g, g+8 of each 16-row tile; dims t, t+4 of each 8-wide k step), pre-split
-  uint32_t qh[2][4][4], ql[2][4][4];
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        const int row = l0 + mt * 16 + g + (e & 1) * 8, col = ks * 8 + t + (e >> 1) * 4;
-        const float x = row < L ? __ldg(qb + static_cast<size_t>(row) * ld_q + col) : 0.f;
-        split_tf32(x, qh[mt][ks][e], ql[mt][ks][e]);
-      }
-  const float scale = rsqrtf(static_cast<float>(kHd));
-  float m_run[2][2], l_run[2][2], oacc[2][4][4];        // per (16-row tile, row half): running max / sum
+  QFrags<HD> qf;                                        // Q fragments, pre-split once (head_dim <= 32)
+  qf.load(qb, ld_q, L, l0, g, t);
+  const float scale = attn_scale<HD>();
+  float m_run[2][2], l_run[2][2], oacc[2][HD / 8][4];   // per (16-row tile, row half): running max / sum
 #pragma unroll
   for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
@@ -1474,7 +1654,7 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
 #pragma unroll
   for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
-    for (int n = 0; n < 4; ++n)
+    for (int n = 0; n < HD / 8; ++n)
 #pragma unroll
       for (int e = 0; e < 4; ++e) oacc[mt][n][e] = 0.f;
 
@@ -1498,15 +1678,18 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
 #pragma unroll
           for (int e = 0; e < 4; ++e) sacc[mt][n][e] = 0.f;
 #pragma unroll
-      for (int ks = 0; ks < 4; ++ks)
+      for (int ks = 0; ks < HD / 8; ++ks) {
+        uint32_t fh[2][4], fl[2][4];
+        qf.step(qb, ld_q, L, l0, g, t, ks, fh, fl);
 #pragma unroll
         for (int n = 0; n < 8; ++n) {
           uint32_t bh0, bl0, bh1, bl1;
           split_tf32(Ks[(n * 8 + g) * kKs + ks * 8 + t], bh0, bl0);
           split_tf32(Ks[(n * 8 + g) * kKs + ks * 8 + t + 4], bh1, bl1);
-          mma_3xtf32(sacc[0][n], qh[0][ks], ql[0][ks], bh0, bh1, bl0, bl1);
-          mma_3xtf32(sacc[1][n], qh[1][ks], ql[1][ks], bh0, bh1, bl0, bl1);
+          mma_3xtf32(sacc[0][n], fh[0], fl[0], bh0, bh1, bl0, bl1);
+          mma_3xtf32(sacc[1][n], fh[1], fl[1], bh0, bh1, bl0, bl1);
         }
+      }
       // softmax step on the fragments: accumulator e -> row (e >> 1) * 8 + g of the tile, column 2t + (e & 1)
 #pragma unroll
       for (int mt = 0; mt < 2; ++mt)
@@ -1540,7 +1723,7 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
           m_run[mt][hf] = m_new;
           l_run[mt][hf] = l_run[mt][hf] * alpha + sum;
 #pragma unroll
-          for (int n = 0; n < 4; ++n) {
+          for (int n = 0; n < HD / 8; ++n) {
             oacc[mt][n][hf * 2] *= alpha;
             oacc[mt][n][hf * 2 + 1] *= alpha;
           }
@@ -1571,7 +1754,7 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
           for (int e = 0; e < 4; ++e)
             split_tf32(Ps[(mt * 16 + g + (e & 1) * 8) * kCkPS + kk * 8 + t + (e >> 1) * 4], ah[mt][e], al[mt][e]);
 #pragma unroll
-        for (int n = 0; n < 4; ++n) {
+        for (int n = 0; n < HD / 8; ++n) {
           uint32_t bh0, bl0, bh1, bl1;
           split_tf32(Vs[(kk * 8 + t) * kVs + n * 8 + g], bh0, bl0);
           split_tf32(Vs[(kk * 8 + t + 4) * kVs + n * 8 + g], bh1, bl1);
@@ -1590,54 +1773,63 @@ attn_chunked_kernel(const float* __restrict__ q, const float* __restrict__ k, co
       const int row = l0 + mt * 16 + hf * 8 + g;
       if (row < L) {
         const float inv = 1.f / l_run[mt][hf];          // l = 0 (every key masked): NaN, like the reference
-        const size_t e0 = (static_cast<size_t>(b) * L + row) * (H * kHd) + h * kHd + 2 * t;
+        const size_t e0 = (static_cast<size_t>(b) * L + row) * (H * HD) + h * HD + 2 * t;
 #pragma unroll
-        for (int n = 0; n < 4; ++n)
+        for (int n = 0; n < HD / 8; ++n)
           attn_store2(out, e0 + n * 8, no_round, oacc[mt][n][hf * 2] * inv, oacc[mt][n][hf * 2 + 1] * inv);
       }
     }
 }
 
+typedef void (*AttnChunkedFn)(const float*, const float*, const float*, const int*, float*, float*, int, int, int, int, int,
+                              int, int);
+
 static int launch_attn_chunked(const float* q, const float* k, const float* v, const int* mask, float* out, float* weights,
-                               int B, int H, int L, int T, int ld_q, int ld_kv, int no_round, int q_per_kv, cudaStream_t st) {
+                               int B, int H, int L, int T, int hd, int ld_q, int ld_kv, int no_round, int q_per_kv,
+                               cudaStream_t st) {
   VQA_REQUIRE(q_per_kv >= 1 && B >= 1 && B % q_per_kv == 0, VQA_E_INVALID, "attn_chunked: the batch must be a multiple of q_per_kv");
   VQA_REQUIRE(L >= 1 && L <= 512 && T >= 1 && T <= 512, VQA_E_INVALID, "attn_chunked: 1..512 queries and 1..512 keys");
   VQA_REQUIRE(weights == nullptr || T <= kChunk, VQA_E_INVALID,
               "attn_chunked: attention weights are stored for at most 64 keys (one chunk)");
+  const int hdi = attn_hd_index(hd);
+  VQA_REQUIRE(hdi >= 0, VQA_E_INVALID, "attn_chunked: head_dim must be 16, 32 or 64");
+  AttnChunkedFn fn = hd == 16 ? &attn_chunked_kernel<16> : hd == 32 ? &attn_chunked_kernel<32> : &attn_chunked_kernel<64>;
   const int qblocks = (L + 31) / 32;
   const int ctas = (qblocks + kCkWarps - 1) / kCkWarps;   // per (pair, head)
   const int warps = (qblocks + ctas - 1) / ctas;          // as few idle warps as the split allows
-  const size_t smem = static_cast<size_t>(kCkSmemFloats - (kCkWarps - warps) * 32 * kCkPS) * sizeof(float);
-  static bool attr_set[kMaxDevices] = {};
+  const size_t smem = static_cast<size_t>(ck_smem_floats(hd) - (kCkWarps - warps) * 32 * kCkPS) * sizeof(float);
+  static bool attr_set[kMaxDevices][3] = {};
   int dev = 0;
   VQA_CUDA_OK(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= kMaxDevices || !attr_set[dev]) {
-    VQA_CUDA_OK(cudaFuncSetAttribute(reinterpret_cast<const void*>(&attn_chunked_kernel),
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize, kCkSmemFloats * static_cast<int>(sizeof(float))));
-    if (dev >= 0 && dev < kMaxDevices) attr_set[dev] = true;
+  if (dev < 0 || dev >= kMaxDevices || !attr_set[dev][hdi]) {
+    VQA_CUDA_OK(cudaFuncSetAttribute(reinterpret_cast<const void*>(fn), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     ck_smem_floats(hd) * static_cast<int>(sizeof(float))));
+    if (dev >= 0 && dev < kMaxDevices) attr_set[dev][hdi] = true;
   }
-  VQA_CUDA_OK(vqa_launch(attn_chunked_kernel, dim3(B * H, ctas), dim3(warps * 32), smem, st, q, k, v, mask, out, weights, H,
+  VQA_CUDA_OK(vqa_launch(fn, dim3(B * H, ctas), dim3(warps * 32), smem, st, q, k, v, mask, out, weights, H,
                          L, T, ld_q, ld_kv, no_round, q_per_kv));
   VQA_LAUNCH_OK("attn_chunked_kernel");
   return VQA_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
-// Fusion tail, one pair per CTA, D = 256 = blockDim (models/fusion.py:299-326, :159-166):
+// Fusion tail, one pair per CTA, D = blockDim (D = 128 .. 512 in steps of 64; models/fusion.py:299-326, :159-166):
 //   phase 1: masked mean pools of the cross-attended and text features (denominator clamp(min=1)),
 //            written as att_pooled / txt_pooled and as the tf32 row [att;txt] of the gate GEMM
 //   phase 2: g = sigmoid(pre) with pre = W[att;txt]+b from that GEMM, g*att+(1-g)*txt, output LayerNorm
 //   phase 0: no gating: att+txt, output LayerNorm (pools computed in place)
-__global__ void __launch_bounds__(256)
+template <int D>
+__global__ void __launch_bounds__(D)
 pool_gate_ln_kernel(const float* __restrict__ xatt, const float* __restrict__ text, const float* __restrict__ mask,
                     const float* __restrict__ pre, const float* __restrict__ gamma, const float* __restrict__ beta,
                     float* __restrict__ fused, float* __restrict__ att_pooled, float* __restrict__ txt_pooled,
                     float* __restrict__ cat, int L, int phase, int no_round, float eps) {
+  static_assert(D % 64 == 0 && D >= 128 && D <= 512, "fusion tail widths: 128 .. 512 in steps of 64");
+  constexpr int NW = D / 32;                            // warps
   pdl_launch_dependents();
   const float gam = __ldg(gamma + threadIdx.x), bet = __ldg(beta + threadIdx.x);   // weights: before the dependency wait
   pdl_wait();
-  constexpr int D = 256;
-  __shared__ float red[16];
+  __shared__ float red[2 * NW];
   const int b = blockIdx.x, d = threadIdx.x;
   const int warp = d >> 5, lane = d & 31;
   float ap, tp;
@@ -1677,23 +1869,39 @@ pool_gate_ln_kernel(const float* __restrict__ xatt, const float* __restrict__ te
   } else {
     f = ap + tp;
   }
-  // block LayerNorm over 256 values (8 warps)
+  // block LayerNorm over D values (D / 32 warps); dividing by D is the multiplication by 1 / D when D is a power of two
   const float s = warp_sum(f);
   if (lane == 0) red[warp] = s;
   __syncthreads();
   float mean = 0.f;
-  for (int w = 0; w < 8; ++w) mean += red[w];
-  const float c = f - mean * (1.f / D);
+  for (int w = 0; w < NW; ++w) mean += red[w];
+  const float c = f - mean / static_cast<float>(D);
   const float q = warp_sum(c * c);
-  if (lane == 0) red[8 + warp] = q;
+  if (lane == 0) red[NW + warp] = q;
   __syncthreads();
   float var = 0.f;
-  for (int w = 0; w < 8; ++w) var += red[8 + w];
-  var *= (1.f / D);
+  for (int w = 0; w < NW; ++w) var += red[NW + w];
+  var /= static_cast<float>(D);
   const float y = c * rsqrtf(var + eps) * gam + bet;
   fused[static_cast<size_t>(b) * D + d] = y;
   if (no_round == 2 && cat != nullptr)   // phases 0 / 2: fp16 copy of the fused feature = operand of the first head Linear
     reinterpret_cast<__half*>(cat)[static_cast<size_t>(b) * D + d] = __float2half_rn(y);
+}
+
+typedef void (*PoolGateLnFn)(const float*, const float*, const float*, const float*, const float*, const float*, float*, float*,
+                             float*, float*, int, int, int, float);
+
+static PoolGateLnFn pool_gate_ln_fn(int D) {
+  switch (D) {
+    case 128: return &pool_gate_ln_kernel<128>;
+    case 192: return &pool_gate_ln_kernel<192>;
+    case 256: return &pool_gate_ln_kernel<256>;
+    case 320: return &pool_gate_ln_kernel<320>;
+    case 384: return &pool_gate_ln_kernel<384>;
+    case 448: return &pool_gate_ln_kernel<448>;
+    case 512: return &pool_gate_ln_kernel<512>;
+    default: return nullptr;
+  }
 }
 
 // softmax over N answers + top-k (k <= 128) in rank_before's order, torch.topk's with ties broken towards the lower index
@@ -1980,7 +2188,11 @@ int run_misc_op(const VqaOp& op, const uint64_t* ext, int n_ext, cudaStream_t st
       return VQA_OK;
     }
     case VQA_OP_LAYERNORM: {
-      VQA_REQUIRE(I[LAYERNORM_I_D] == 256, VQA_E_INVALID, "layernorm: D must be 256");
+      const int D = I[LAYERNORM_I_D];
+      const LayerNormFn fn = layernorm_fn(D);
+      VQA_REQUIRE(fn != nullptr, VQA_E_INVALID, "layernorm: D must be 128 .. 512 in steps of 64");
+      VQA_REQUIRE(D == 256 || (I[LAYERNORM_I_ld_src] >= D && I[LAYERNORM_I_ld_src] % 4 == 0), VQA_E_ALIGN,
+                  "layernorm: the source row pitch must be a multiple of 4 floats, at least D");
       const int rows = I[LAYERNORM_I_rows];
       LnExtra ex;
       ex.gamma2 = PTR(const float*, LAYERNORM_P_gamma2); ex.beta2 = PTR(const float*, LAYERNORM_P_beta2);
@@ -1990,38 +2202,39 @@ int run_misc_op(const VqaOp& op, const uint64_t* ext, int n_ext, cudaStream_t st
       VQA_REQUIRE((ex.gamma2 == nullptr || (ex.beta2 != nullptr && ex.dst2 != nullptr)) &&
                       (ex.gamma3 == nullptr || (ex.beta3 != nullptr && ex.dst3 != nullptr)),
                   VQA_E_INVALID, "layernorm: a chained LayerNorm needs gamma, beta and an output");
-      VQA_CUDA_OK(vqa_launch(layernorm256_kernel, dim3(blocks_for(rows, 8)), dim3(256), 0, st, 
+      VQA_CUDA_OK(vqa_launch(fn, dim3(blocks_for(rows, 8)), dim3(256), 0, st, 
           PTR(const float*, LAYERNORM_P_src), PTR(const float*, LAYERNORM_P_gamma), PTR(const float*, LAYERNORM_P_beta),
           PTR(float*, LAYERNORM_P_dst), PTR(const float*, LAYERNORM_P_pos), rows, I[LAYERNORM_I_ld_src],
           I[LAYERNORM_I_mode], I[LAYERNORM_I_round_tf32], I[LAYERNORM_I_S], I[LAYERNORM_I_Pg], I[LAYERNORM_I_RPIg],
           op.f[LAYERNORM_F_eps], ex));
-      VQA_LAUNCH_OK("layernorm256_kernel");
+      VQA_LAUNCH_OK(D == 256 ? "layernorm256_kernel" : "layernorm_kernel");
       return VQA_OK;
     }
     case VQA_OP_SELF_ATTN: {
       const int L = I[SELF_ATTN_I_L], H = I[SELF_ATTN_I_H], B = I[SELF_ATTN_I_B];
-      VQA_REQUIRE(L >= 1 && L <= 64 && I[SELF_ATTN_I_hd] == kHd, VQA_E_INVALID, "self_attn: L<=64, head_dim=32");
+      const int hd = I[SELF_ATTN_I_hd];
+      VQA_REQUIRE(L >= 1 && L <= 64 && attn_hd_index(hd) >= 0, VQA_E_INVALID, "self_attn: L<=64, head_dim 16, 32 or 64");
       const float* qkv = PTR(const float*, SELF_ATTN_P_qkv);
-      const int D = H * kHd, ld = I[SELF_ATTN_I_ld_qkv];
+      const int D = H * hd, ld = I[SELF_ATTN_I_ld_qkv];
       VQA_REQUIRE(ld % 4 == 0 && (reinterpret_cast<uintptr_t>(qkv) & 15) == 0, VQA_E_ALIGN, "self_attn: qkv alignment");
       VQA_REQUIRE((reinterpret_cast<uintptr_t>(PTR(float*, SELF_ATTN_P_out)) & 15) == 0, VQA_E_ALIGN, "self_attn: out alignment");
       return launch_attn(qkv, qkv + D, qkv + 2 * D, PTR(const int*, SELF_ATTN_P_mask), PTR(float*, SELF_ATTN_P_out), nullptr, B,
-                         H, L, L, ld, ld, I[SELF_ATTN_I_no_round], 1, st);
+                         H, L, L, hd, ld, ld, I[SELF_ATTN_I_no_round], 1, st);
     }
     case VQA_OP_CROSS_ATTN: {
       const int L = I[CROSS_ATTN_I_L], T = I[CROSS_ATTN_I_T], H = I[CROSS_ATTN_I_H], B = I[CROSS_ATTN_I_B];
-      VQA_REQUIRE(L >= 1 && L <= 64 && T >= 1 && T <= 64 && I[CROSS_ATTN_I_hd] == kHd, VQA_E_INVALID,
-                  "cross_attn: L<=64, T<=64, head_dim=32");
+      VQA_REQUIRE(L >= 1 && L <= 64 && T >= 1 && T <= 64 && attn_hd_index(I[CROSS_ATTN_I_hd]) >= 0, VQA_E_INVALID,
+                  "cross_attn: L<=64, T<=64, head_dim 16, 32 or 64");
       const float* kv = PTR(const float*, CROSS_ATTN_P_kv);
       VQA_REQUIRE(I[CROSS_ATTN_I_ld_q] % 4 == 0 && I[CROSS_ATTN_I_ld_kv] % 4 == 0 && I[CROSS_ATTN_I_k_off] % 4 == 0 &&
                       I[CROSS_ATTN_I_v_off] % 4 == 0, VQA_E_ALIGN, "cross_attn: leading dimensions must be multiples of 4");
       return launch_attn(PTR(const float*, CROSS_ATTN_P_q), kv + I[CROSS_ATTN_I_k_off], kv + I[CROSS_ATTN_I_v_off], nullptr,
-                         PTR(float*, CROSS_ATTN_P_out), PTR(float*, CROSS_ATTN_P_weights), B, H, L, T, I[CROSS_ATTN_I_ld_q],
+                         PTR(float*, CROSS_ATTN_P_out), PTR(float*, CROSS_ATTN_P_weights), B, H, L, T, I[CROSS_ATTN_I_hd], I[CROSS_ATTN_I_ld_q],
                          I[CROSS_ATTN_I_ld_kv], I[CROSS_ATTN_I_no_round], I[CROSS_ATTN_I_q_per_kv] > 0 ? I[CROSS_ATTN_I_q_per_kv] : 1, st);
     }
     case VQA_OP_ATTN_CHUNKED: {
       const int L = I[ATTN_CHUNKED_I_L], T = I[ATTN_CHUNKED_I_T], H = I[ATTN_CHUNKED_I_H], B = I[ATTN_CHUNKED_I_B];
-      VQA_REQUIRE(I[ATTN_CHUNKED_I_hd] == kHd && H >= 1, VQA_E_INVALID, "attn_chunked: head_dim=32");
+      VQA_REQUIRE(attn_hd_index(I[ATTN_CHUNKED_I_hd]) >= 0 && H >= 1, VQA_E_INVALID, "attn_chunked: head_dim 16, 32 or 64");
       const float* kv = PTR(const float*, ATTN_CHUNKED_P_kv);
       VQA_REQUIRE(I[ATTN_CHUNKED_I_ld_q] % 4 == 0 && I[ATTN_CHUNKED_I_ld_kv] % 4 == 0 && I[ATTN_CHUNKED_I_k_off] % 4 == 0 &&
                       I[ATTN_CHUNKED_I_v_off] % 4 == 0 && (reinterpret_cast<uintptr_t>(kv) & 15) == 0 &&
@@ -2029,19 +2242,21 @@ int run_misc_op(const VqaOp& op, const uint64_t* ext, int n_ext, cudaStream_t st
                   VQA_E_ALIGN, "attn_chunked: K / V and the output must be 16-byte aligned, leading dimensions multiples of 4");
       return launch_attn_chunked(PTR(const float*, ATTN_CHUNKED_P_q), kv + I[ATTN_CHUNKED_I_k_off], kv + I[ATTN_CHUNKED_I_v_off],
                                  PTR(const int*, ATTN_CHUNKED_P_mask), PTR(float*, ATTN_CHUNKED_P_out),
-                                 PTR(float*, ATTN_CHUNKED_P_weights), B, H, L, T, I[ATTN_CHUNKED_I_ld_q], I[ATTN_CHUNKED_I_ld_kv],
+                                 PTR(float*, ATTN_CHUNKED_P_weights), B, H, L, T, I[ATTN_CHUNKED_I_hd], I[ATTN_CHUNKED_I_ld_q], I[ATTN_CHUNKED_I_ld_kv],
                                  I[ATTN_CHUNKED_I_no_round], I[ATTN_CHUNKED_I_q_per_kv], st);
     }
     case VQA_OP_POOL_GATE_LN: {
       const int phase = I[POOL_GATE_LN_I_phase];
-      VQA_REQUIRE(I[POOL_GATE_LN_I_D] == 256, VQA_E_INVALID, "pool_gate_ln: D must be 256");
+      const int D = I[POOL_GATE_LN_I_D];
+      const PoolGateLnFn fn = pool_gate_ln_fn(D);
+      VQA_REQUIRE(fn != nullptr, VQA_E_INVALID, "pool_gate_ln: D must be 128 .. 512 in steps of 64");
       VQA_REQUIRE(phase >= 0 && phase <= 2 && (phase != 0 || I[POOL_GATE_LN_I_use_gate] == 0), VQA_E_INVALID,
                   "pool_gate_ln: gating runs as pool -> gate GEMM -> mix (phases 1, 2)");
       VQA_REQUIRE(PTR(float*, POOL_GATE_LN_P_att_pooled) && PTR(float*, POOL_GATE_LN_P_txt_pooled), VQA_E_INVALID,
                   "pool_gate_ln: pooled buffers are required");
       VQA_REQUIRE(phase != 1 || PTR(float*, POOL_GATE_LN_P_cat), VQA_E_INVALID, "pool_gate_ln: phase 1 needs cat");
       VQA_REQUIRE(phase != 2 || PTR(const float*, POOL_GATE_LN_P_pre), VQA_E_INVALID, "pool_gate_ln: phase 2 needs pre");
-      VQA_CUDA_OK(vqa_launch(pool_gate_ln_kernel, dim3(I[POOL_GATE_LN_I_B]), dim3(256), 0, st,
+      VQA_CUDA_OK(vqa_launch(fn, dim3(I[POOL_GATE_LN_I_B]), dim3(D), 0, st,
           PTR(const float*, POOL_GATE_LN_P_xatt), PTR(const float*, POOL_GATE_LN_P_text),
           PTR(const float*, POOL_GATE_LN_P_mask), PTR(const float*, POOL_GATE_LN_P_pre),
           PTR(const float*, POOL_GATE_LN_P_gamma), PTR(const float*, POOL_GATE_LN_P_beta),

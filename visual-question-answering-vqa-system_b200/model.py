@@ -19,9 +19,18 @@ import torch.nn.functional as F
 
 from .modules import AnswerHead, CustomResNet, MultimodalFusion, TransformerTextEncoder
 
-_SUPPORTED = ("The sm_100a engine is specialised for embed_dim=256, 8 heads, ffn_hidden_dim=1024 "
-              "(the reference defaults); layer counts, vocab/answer sizes, max_question_length<=512 "
-              "and the SE/spatial/gating ablation switches are free.")
+_SUPPORTED = ("The sm_100a engine runs embed_dim 128..512 in steps of 64 with head_dim = embed_dim / num_attention_heads "
+              "in {16, 32, 64} and ffn_hidden_dim 64..4096 in steps of 64 (the reference defaults are 256 / 8 heads / 1024); "
+              "layer counts, vocab/answer sizes, max_question_length<=512 and the SE/spatial/gating ablation switches are free.")
+
+
+def supported_config(embed_dim: int, num_attention_heads: int, ffn_hidden_dim: int, max_question_length: int) -> bool:
+    """Whether the engine has kernels for these widths (``_SUPPORTED``).  embed_dim is the K of the text and fusion
+    Linears (32-element chunks of the tf32 GEMM, 64-element chunks of the fp16 ones) and the width of the LayerNorm and
+    fusion-tail kernels; head_dim selects the attention kernels' instantiation; the cross-attention FFN is 4 * embed_dim."""
+    D, H, F = embed_dim, num_attention_heads, ffn_hidden_dim
+    return (D % 64 == 0 and 128 <= D <= 512 and H >= 1 and D % H == 0 and D // H in (16, 32, 64)
+            and F % 64 == 0 and 64 <= F <= 4096 and max_question_length <= 512)
 
 
 class VQAModel(nn.Module):
@@ -61,9 +70,7 @@ class VQAModel(nn.Module):
     # ------------------------------------------------------------------ engine plumbing
     def _check_supported(self):
         c = self.config
-        if c["embed_dim"] != 256 or c["num_attention_heads"] != 8 or c["ffn_hidden_dim"] != 1024:
-            raise NotImplementedError(_SUPPORTED)
-        if c["max_question_length"] > 512:
+        if not supported_config(c["embed_dim"], c["num_attention_heads"], c["ffn_hidden_dim"], c["max_question_length"]):
             raise NotImplementedError(_SUPPORTED)
 
     def engine(self):

@@ -386,7 +386,9 @@ def build_weights(sd: Dict[str, torch.Tensor], cfg: dict, device, precision: str
     # ---- text encoder (fp32 storage, tf32-rounded GEMM operands)
     t = "text_encoder"
     D = cfg["embed_dim"]
-    W.add("text.emb", sd[t + ".token_embedding.weight"].float() * math.sqrt(D), f32)  # exact: sqrt(256)=16
+    # the reference scales after the lookup (F.embedding(ids, emb) * math.sqrt(D)); both are the same fp32 product of each
+    # table element and fp32(sqrt(D)), so scaling the table once gives the same bits for every D, a perfect square or not
+    W.add("text.emb", sd[t + ".token_embedding.weight"].float() * math.sqrt(D), f32)
     W.add("text.pe", sd[t + ".positional_encoding.pe"][0], f32)
     layer = 0
     while f"{t}.layers.{layer}.norm1.weight" in sd:
@@ -580,6 +582,10 @@ class OpList:
                     pair = False
                 elif step == "bn" and bn > 64 and npad % 64 == 0:
                     bn = 64
+        # widths that are multiples of 64 but not of the chosen tile (embed_dim 192, 320, 448 and their multiples, FFN
+        # widths such as 320): the largest tile that divides the weight rows
+        while npad % bn and bn > 64 and sf == 1 and topk is None:
+            bn //= 2
         assert npad % bn == 0 and npad >= N, (name, npad, bn)
         assert len(groups) <= MAX_GROUPS and MT * bn * sf <= 512
         assert sf == 1 or (1 < sf <= 3 and npad == sf * bn and MT == 1 and pool_to is None and (sf - 1) * sf_step <= 4)
@@ -719,9 +725,10 @@ class OpList:
             p.update({f"gamma{k}": self.W.buf(g2), f"beta{k}": self.W.buf(b2), f"dst{k}": dst2})
         return i, p
 
-    def layernorm(self, name, src, g, b, dst, rows, rnd=False, ld=256, extra=()):
+    def layernorm(self, name, src, g, b, dst, rows, rnd=False, ld=None, extra=()):
+        D = self.W.items[g][2][0]        # the width of the norm is that of its gamma
         xi, xp = self._ln_extra(extra)
-        self._op("layernorm", name, dict(rows=rows, D=256, ld_src=ld, mode=0, round_tf32=self._ln_mode(rnd), S=0, Pg=0, RPIg=0, **xi),
+        self._op("layernorm", name, dict(rows=rows, D=D, ld_src=ld or D, mode=0, round_tf32=self._ln_mode(rnd), S=0, Pg=0, RPIg=0, **xi),
                  dict(src=src, gamma=self.W.buf(g), beta=self.W.buf(b), dst=dst, pos=None, **xp), dict(eps=1e-5))
 
 
@@ -1031,7 +1038,10 @@ class Program(OpList):
         qkv = self._buf("text.qkv", f32, T, 3 * D)
         ctx = self._buf("text.ctx", self.tdt, T, D)
         chain = self.chain and D == 256 and F % 128 == 0 and F <= 1024
-        hid = None if chain else self._buf("text.hid", self.tdt, T, F)    # the chain kernels keep the FFN hidden state on chip
+        # FFN hidden state of the text layers (F) and of the cross-attention layers (4 * D, modules.py:203), one buffer for
+        # both; the chain kernels keep it on chip
+        Fx = W.items["x.0.fc1.w"][2][0] if n_layers else F
+        hid = None if chain else self._buf("text.hid", self.tdt, T, max(F, Fx))
         V = W.items["text.emb"][2][0]
         if fuse_embed:   # embedding + position, the first layer's LayerNorm and the mask normalisation in one launch
             self._op("embed", "text.embed", dict(B=B, L=L, D=D, V=V, round_tf32=self._ln_mode(True), mask_dtype=self.mask_dtype),
@@ -1146,8 +1156,8 @@ class Program(OpList):
             # q = src_q + W_o ctx   (first layer reads the text features as residual, writes the stream buffer)
             self.linear(p + ".o", cx, T, D, p + ".o.w", None, q, D, res=src_q)
             self.layernorm(p + ".lnf", q, p + ".lnf.g", p + ".lnf.b", qn, T, rnd=True)
-            self.linear(p + ".fc1", qn, T, D, p + ".fc1.w", p + ".fc1.b", hid, F, relu=True, rnd=True)
-            self.linear(p + ".fc2", hid, T, F, p + ".fc2.w", p + ".fc2.b", q, D, res=q)
+            self.linear(p + ".fc1", qn, T, D, p + ".fc1.w", p + ".fc1.b", hid, Fx, relu=True, rnd=True)
+            self.linear(p + ".fc2", hid, T, Fx, p + ".fc2.w", p + ".fc2.b", q, D, res=q)
             src_q = q
         fused = self._buf("fused", f32, B, D)
         attp = self._buf("attended_pooled", f32, B, D)
