@@ -477,7 +477,7 @@ def make_case(ctor, B, L=None, in_fmt="nchw_f32", mask_kind="i64", precision="bf
     cfg = model.config
     L = L or (ids.shape[1] if ids is not None else cfg["max_question_length"])
     Bi = B if n_images is None else n_images
-    u8, img, sids, smask = synth_batch(B, seed, max_len=L, vocab=cfg["vocab_size"])
+    u8, img, sids, smask = synth_batch(B, seed, max_len=L, vocab=max(cfg["vocab_size"], 5))   # seeded ids lie in [4, V)
     images = (u8 if in_fmt == "hwc_u8" else img)[:Bi]
     if ids is None:
         ids = sids

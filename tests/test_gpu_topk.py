@@ -27,9 +27,8 @@ def _check_probs(tag, got_i, got_p, logits):
     return worst
 
 
-def _run_softmax_topk(logits, k):
-    """One softmax_topk op through an OpList / Plan, on ``logits`` [B, N] (fp32, CPU)."""
-    B, N = logits.shape
+def _topk_plan(B, N, k):
+    """A Plan of one softmax_topk op over the logits / top_idx / top_probs slots."""
     W = P.Weights("cuda")
     W.add("unused", torch.zeros(4), torch.float32)
     W.finalize()
@@ -37,9 +36,19 @@ def _run_softmax_topk(logits, k):
     ol._op("softmax_topk", "topk", dict(B=B, N=N, k=k, ld=N),
            dict(logits=P.ExtRef(P.EXT["logits"]), idx=P.ExtRef(P.EXT["top_idx"]), probs=P.ExtRef(P.EXT["top_probs"])))
     ol.commit()
-    ext = [None, None, None, logits.cuda(), torch.full((B, k), -7, dtype=torch.int64, device="cuda"),
-           torch.full((B, k), -7.0, device="cuda")]
-    plan = Plan(ol.ops, 0)
+    return Plan(ol.ops, 0)
+
+
+def _topk_ext(logits, k):
+    B = logits.shape[0]
+    return [None, None, None, logits.cuda(), torch.full((B, k), -7, dtype=torch.int64, device="cuda"),
+            torch.full((B, k), -7.0, device="cuda")]
+
+
+def _run_softmax_topk(logits, k):
+    """One softmax_topk op through an OpList / Plan, on ``logits`` [B, N] (fp32, CPU)."""
+    plan = _topk_plan(*logits.shape, k)
+    ext = _topk_ext(logits, k)
     plan.run([0 if t is None else t.data_ptr() for t in ext], torch.cuda.current_stream().cuda_stream)
     torch.cuda.synchronize()
     return ext[4], ext[5]
@@ -59,12 +68,20 @@ def test_softmax_topk_kernel_is_exact_on_every_row_kind(N, k):
     _check_probs(f"softmax_topk N={N} k={k}", idx, probs, logits)
 
 
-def test_softmax_topk_launcher_rejects_bad_sizes():
-    """k = 129, k > N and N = 10 001 are refused before anything is launched."""
-    for N, k in ((300, 129), (8, 9), (10001, 5)):
-        logits = torch.randn(2, N)
-        with pytest.raises(VqaError):
-            _run_softmax_topk(logits, k)
+def test_softmax_topk_launcher_refuses_bad_sizes_and_heads_over_50000():
+    """k = 129, k > N and N = 50 001 (one above the largest row the kernel keeps in shared memory) are refused, nothing
+    is launched and the outputs are not written."""
+    from vqa_b200.runtime import launch_count
+    for N, k in ((300, 129), (8, 9), (50001, 5)):
+        plan = _topk_plan(2, N, k)
+        ext = _topk_ext(torch.randn(2, N), k)
+        torch.cuda.synchronize()
+        n0 = launch_count()
+        with pytest.raises(VqaError, match="N<=50000"):
+            plan.run([0 if t is None else t.data_ptr() for t in ext], torch.cuda.current_stream().cuda_stream)
+        torch.cuda.synchronize()
+        assert launch_count() == n0, f"N={N} k={k}: a kernel was launched"
+        assert bool((ext[4] == -7).all()) and bool((ext[5] == -7.0).all()), f"N={N} k={k}: the outputs were written"
 
 
 def test_model_top_k_paths_agree_with_the_fp64_reference(monkeypatch):

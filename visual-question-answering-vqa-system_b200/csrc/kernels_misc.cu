@@ -690,8 +690,8 @@ stage_tail_kernel(const StageTailParams p) {
   float* red = reinterpret_cast<float*>(tile + static_cast<size_t>(NP) * C8 * Vec::N);   // [red_rows][C]; later mx/av maps
   float* part = red + red_rows * C;                     // [C] this CTA's channel sums (read by the cluster)
   float* sc = part + C;                                 // [C] SE scale
-  float* hid = sc + C;                                  // [R]
-  float* att = hid + 256;                               // [NP] spatial attention (CS == 1)
+  float* hid = sc + C;                                  // [max(R, 256)]: the floor keeps the default's layout
+  float* att = hid + (p.R > 256 ? p.R : 256);           // [NP] spatial attention (CS == 1)
   float* wc = att + NP;                                 // [2*ks*ks] spatial conv weights
   const bool use_se = p.w1 != nullptr;
 
@@ -1967,6 +1967,9 @@ __global__ void softmax_topk_kernel(const float* __restrict__ logits, long long*
   }
 }
 
+constexpr int kSoftmaxTopKMaxN = 50000;
+inline size_t softmax_topk_smem(int N) { return (static_cast<size_t>(N) + 64 + (N + 31) / 32) * sizeof(float); }
+
 inline unsigned blocks_for(long long n, int threads) { return static_cast<unsigned>((n + threads - 1) / threads); }
 
 }  // namespace
@@ -2084,7 +2087,8 @@ int run_misc_op(const VqaOp& op, const uint64_t* ext, int n_ext, cudaStream_t st
       VQA_REQUIRE(q.H % q.CS == 0 && (!q.mode || (q.H / q.CS) % 2 == 0) && (!q.mode || q.W % 2 == 0), VQA_E_INVALID,
                   "stage_tail: rows per CTA must be whole (and even for the phase split)");
       VQA_REQUIRE(q.wconv == nullptr || q.CS == 1, VQA_E_INVALID, "stage_tail: spatial attention needs the whole image (CS = 1)");
-      VQA_REQUIRE(q.R <= 256 && (q.w1 == nullptr) == (q.w2 == nullptr), VQA_E_INVALID, "stage_tail: SE hidden width > 256");
+      VQA_REQUIRE(q.R >= 0 && q.R <= C && (q.w1 == nullptr) == (q.w2 == nullptr), VQA_E_INVALID,
+                  "stage_tail: SE hidden width must be at most the channel count");
       VQA_REQUIRE(q.Po > 0 && q.RPIo % q.Po == 0, VQA_E_INVALID, "stage_tail: bad destination grid");
       const int NP = q.H / q.CS * q.W, lanes = kTailThreads / q.C8;
       const int part_rows = lanes / (q.C8 < 32 ? 32 / q.C8 : 1);
@@ -2116,7 +2120,8 @@ int run_misc_op(const VqaOp& op, const uint64_t* ext, int n_ext, cudaStream_t st
           return VQA_OK;
         }
       }
-      const size_t smem = static_cast<size_t>(NP) * C * (f32 ? 4 : 2) + sizeof(float) * (static_cast<size_t>(red_rows) * C + 2 * C + 256 + NP + 128);
+      const size_t hid_floats = q.R > 256 ? q.R : 256;
+      const size_t smem = static_cast<size_t>(NP) * C * (f32 ? 4 : 2) + sizeof(float) * (static_cast<size_t>(red_rows) * C + 2 * C + hid_floats + NP + 128);
       VQA_REQUIRE(smem <= 227 * 1024, VQA_E_INVALID, "stage_tail: rows per CTA exceed shared memory (raise CS)");
       static bool attr_set[kMaxDevices] = {};   // per device: the attribute belongs to the device's context
       int dev = 0;
@@ -2268,8 +2273,19 @@ int run_misc_op(const VqaOp& op, const uint64_t* ext, int n_ext, cudaStream_t st
     }
     case VQA_OP_SOFTMAX_TOPK: {
       const int N = I[SOFTMAX_TOPK_I_N], k = I[SOFTMAX_TOPK_I_k];
-      VQA_REQUIRE(k >= 1 && k <= 128 && k <= N && N <= 10000, VQA_E_INVALID, "softmax_topk: 1<=k<=min(128, N), N<=10000");
-      VQA_CUDA_OK(vqa_launch(softmax_topk_kernel, dim3(I[SOFTMAX_TOPK_I_B]), dim3(256), (N + 64 + (N + 31) / 32) * sizeof(float), st, 
+      VQA_REQUIRE(k >= 1 && k <= 128 && k <= N && N <= kSoftmaxTopKMaxN, VQA_E_INVALID,
+                  "softmax_topk: 1<=k<=min(128, N), N<=50000");
+      // the row lives in shared memory: up to 206 KB at 50 000 answers, beyond the default 48 KB
+      static bool attr_set[kMaxDevices] = {};   // per device: the attribute belongs to the device's context
+      int dev = 0;
+      VQA_CUDA_OK(cudaGetDevice(&dev));
+      if (dev < 0 || dev >= kMaxDevices || !attr_set[dev]) {
+        VQA_CUDA_OK(cudaFuncSetAttribute(reinterpret_cast<const void*>(&softmax_topk_kernel),
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         static_cast<int>(softmax_topk_smem(kSoftmaxTopKMaxN))));
+        if (dev >= 0 && dev < kMaxDevices) attr_set[dev] = true;
+      }
+      VQA_CUDA_OK(vqa_launch(softmax_topk_kernel, dim3(I[SOFTMAX_TOPK_I_B]), dim3(256), softmax_topk_smem(N), st,
           PTR(const float*, SOFTMAX_TOPK_P_logits), PTR(long long*, SOFTMAX_TOPK_P_idx),
           PTR(float*, SOFTMAX_TOPK_P_probs), N, k, I[SOFTMAX_TOPK_I_ld]));
       VQA_LAUNCH_OK("softmax_topk_kernel");

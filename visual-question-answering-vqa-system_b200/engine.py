@@ -19,14 +19,16 @@ class ImageCache:
     """Question-independent half of the forward for ``n_images`` images: K/V of every cross-attention layer
     (``kv[l]`` fp32 ``[n_images, 49, 2 * embed_dim]``, K in the first embed_dim columns).  The reference recomputes these
     per (image, question) pair (models/fusion.py:284, models/cross_attention.py:160-161,286-287); ``Engine.encode_images``
-    computes them once and ``Engine.answer`` runs only the question side against them."""
+    computes them once and ``Engine.answer`` runs only the question side against them.  A model without cross-attention
+    layers caches nothing but the number of images."""
 
-    def __init__(self, kv):
+    def __init__(self, kv, n_images: Optional[int] = None):
         self.kv = list(kv)
-
-    @property
-    def n_images(self) -> int:
-        return int(self.kv[0].shape[0]) if self.kv else 0
+        if n_images is None:
+            if not self.kv:
+                raise ValueError("an ImageCache without K/V tensors needs n_images")
+            n_images = int(self.kv[0].shape[0])
+        self.n_images = int(n_images)
 
     @property
     def nbytes(self) -> int:
@@ -34,16 +36,26 @@ class ImageCache:
 
     def select(self, index) -> "ImageCache":
         """Cache rows ``index`` (LongTensor / list, repeats allowed): one entry per question for ``Engine.answer``."""
-        idx = torch.as_tensor(index, dtype=torch.long, device=self.kv[0].device)
-        return ImageCache([t.index_select(0, idx) for t in self.kv])
+        idx = torch.as_tensor(index, dtype=torch.long, device=self.kv[0].device if self.kv else "cpu").reshape(-1)
+        return ImageCache([t.index_select(0, idx) for t in self.kv], int(idx.numel()))
 
     @staticmethod
     def cat(caches) -> "ImageCache":
         caches = list(caches)
-        return ImageCache([torch.cat([c.kv[l] for c in caches], 0) for l in range(len(caches[0].kv))])
+        return ImageCache([torch.cat([c.kv[l] for c in caches], 0) for l in range(len(caches[0].kv))],
+                          sum(c.n_images for c in caches))
 
 
 MAX_TOP_K = 128      # softmax_topk_kernel selects one winner per block-wide pass
+MAX_TOP_K_ANSWERS = 50000   # softmax_topk_kernel keeps a row of logits in shared memory (206 KB at 50 000)
+
+
+def check_cacheable(cfg: dict):
+    """The question-side program reads each cached layer's K/V from its own external slot: one per layer, up to
+    ``program.MAX_CACHED_LAYERS``."""
+    if cfg["num_cross_layers"] > P.MAX_CACHED_LAYERS:
+        raise NotImplementedError(f"the image cache holds up to {P.MAX_CACHED_LAYERS} cross-attention layers, the model "
+                                  f"has {cfg['num_cross_layers']}: use forward / predict")
 
 
 class Engine:
@@ -74,6 +86,9 @@ class Engine:
         n_images = n_images or B
         if top_k < 0 or top_k > min(MAX_TOP_K, self.cfg["num_answers"]):
             raise ValueError(f"top_k must be between 1 and min({MAX_TOP_K}, num_answers={self.cfg['num_answers']}), got {top_k}")
+        if top_k and self.cfg["num_answers"] > MAX_TOP_K_ANSWERS:
+            raise ValueError(f"top-k selection runs for at most {MAX_TOP_K_ANSWERS} answers, the model has "
+                             f"{self.cfg['num_answers']}: call forward and select from the logits")
         key = (B, L, in_fmt, mask_dtype, want_aux, top_k, self.window, n_images, side, slot)
         hit = self._plans.get(key)
         if hit is not None:
@@ -147,7 +162,7 @@ class Engine:
         if not torch.cuda.is_current_stream_capturing():
             images.record_stream(stream)
         D2 = 2 * self.cfg["embed_dim"]
-        return ImageCache([prog.tensor(f"x.{l}.kv").view(Bi, 49, D2).clone() for l in range(prog.n_cross_layers)])
+        return ImageCache([prog.tensor(f"x.{l}.kv").view(Bi, 49, D2).clone() for l in range(prog.n_cross_layers)], Bi)
 
     def answer(self, cache: ImageCache, token_ids: torch.Tensor, attention_mask: Optional[torch.Tensor] = None,
                top_k: int = 0):

@@ -86,6 +86,9 @@ class VQAInference:
             self.model = VQAModel(vocab_size=DEFAULT_QUESTION_VOCAB_SIZE,
                                   num_answers=DEFAULT_NUM_ANSWERS).to(self.device)
         self.model.eval()
+        if self.image_cache_size > 0:
+            from .engine import check_cacheable
+            check_cacheable(self.model.config)
         if os.path.exists(self.question_vocab_path):
             self.tokenizer = Tokenizer()
             self.tokenizer.load(self.question_vocab_path)
@@ -383,7 +386,7 @@ class VQAInference:
                  "h_probs": torch.empty(B, k, dtype=torch.float32).pin_memory(),
                  "d_ids": torch.zeros(B, L, dtype=torch.long, device=dev),
                  "d_mask": torch.ones(B, L, dtype=torch.long, device=dev)}
-            static = ImageCache(g["kv"])
+            static = ImageCache(g["kv"], cache.n_images)
             engine = self.model.engine()
             for _ in range(2):       # warm up: builds the plan, loads kernels
                 engine.answer(static, g["d_ids"], g["d_mask"], top_k=k)

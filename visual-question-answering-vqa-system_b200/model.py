@@ -21,7 +21,10 @@ from .modules import AnswerHead, CustomResNet, MultimodalFusion, TransformerText
 
 _SUPPORTED = ("The sm_100a engine runs embed_dim 128..512 in steps of 64 with head_dim = embed_dim / num_attention_heads "
               "in {16, 32, 64} and ffn_hidden_dim 64..4096 in steps of 64 (the reference defaults are 256 / 8 heads / 1024); "
-              "layer counts, vocab/answer sizes, max_question_length<=512 and the SE/spatial/gating ablation switches are free.")
+              "max_question_length is at most 512.  Layer counts (0 included), vocab sizes, answer counts, se_reduction and "
+              "the SE/spatial/gating ablation switches are free, with two limits: top-k selection (predict, VQAInference) "
+              "runs for at most 50000 answers (forward has no limit), and the image cache (encode_images / answer, "
+              "VQAInference(image_cache_size>0)) holds at most 8 cross-attention layers.")
 
 
 def supported_config(embed_dim: int, num_attention_heads: int, ffn_hidden_dim: int, max_question_length: int) -> bool:
@@ -118,6 +121,8 @@ class VQAModel(nn.Module):
         ``ImageCache`` that can be kept across calls.  ``answer(cache, ids, mask)`` then equals ``forward`` bit for bit."""
         if self.training:
             raise NotImplementedError("eval-mode inference path only; call .eval()")
+        from .engine import check_cacheable
+        check_cacheable(self.config)
         with torch.no_grad():
             return self.engine().encode_images(images)
 

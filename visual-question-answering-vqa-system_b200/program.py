@@ -1033,15 +1033,18 @@ class Program(OpList):
             if not fuse_embed:
                 self._op("mask_prep", "mask", dict(B=B, L=L, dtype=self.mask_dtype),
                          dict(src=ExtRef(EXT["mask"]), dst=mask, dstf=maskw))
+        n_text = 0
+        while f"text.{n_text}.qkv.w" in W:
+            n_text += 1
         xt = self._buf("text.x", f32, T, D)
-        xn = self._buf("text.xn", self.tdt, T, D)
-        qkv = self._buf("text.qkv", f32, T, 3 * D)
-        ctx = self._buf("text.ctx", self.tdt, T, D)
+        xn = self._buf("text.xn", self.tdt, T, D) if n_text else None
+        qkv = self._buf("text.qkv", f32, T, 3 * D) if n_text else None
+        ctx = self._buf("text.ctx", self.tdt, T, D) if n_text else None
         chain = self.chain and D == 256 and F % 128 == 0 and F <= 1024
         # FFN hidden state of the text layers (F) and of the cross-attention layers (4 * D, modules.py:203), one buffer for
         # both; the chain kernels keep it on chip
         Fx = W.items["x.0.fc1.w"][2][0] if n_layers else F
-        hid = None if chain else self._buf("text.hid", self.tdt, T, max(F, Fx))
+        hid = None if chain or not (n_text or n_layers) else self._buf("text.hid", self.tdt, T, max(F, Fx))
         V = W.items["text.emb"][2][0]
         if fuse_embed:   # embedding + position, the first layer's LayerNorm and the mask normalisation in one launch
             self._op("embed", "text.embed", dict(B=B, L=L, D=D, V=V, round_tf32=self._ln_mode(True), mask_dtype=self.mask_dtype),
@@ -1089,10 +1092,12 @@ class Program(OpList):
         # projected image); the main lane runs projector -> K/V of layer 0 -> attention / FFN chain and joins the
         # side lane right before each attention.  Ops are issued in list order, so a JOIN waits only for what
         # precedes it in the list.
-        q = self._buf("x.q", f32, T, D)          # running query (residual stream)
-        qn = None if chain else self._buf("x.qn", self.tdt, T, D)   # chains: each layer's kernel normalises the next query
-        qp = self._buf("x.qp", f32, T, D)
-        cx = self._buf("x.ctx", self.tdt, T, D)
+        q = qn = qp = cx = None
+        if n_layers:
+            q = self._buf("x.q", f32, T, D)          # running query (residual stream)
+            qn = None if chain else self._buf("x.qn", self.tdt, T, D)   # chains: each layer's kernel normalises the next query
+            qp = self._buf("x.qp", f32, T, D)
+            cx = self._buf("x.ctx", self.tdt, T, D)
         if cached:
             imns, kvs = [], [ExtRef(EXT[f"kv{l}"]) for l in range(n_layers)]
         else:
@@ -1159,6 +1164,9 @@ class Program(OpList):
             self.linear(p + ".fc1", qn, T, D, p + ".fc1.w", p + ".fc1.b", hid, Fx, relu=True, rnd=True)
             self.linear(p + ".fc2", hid, T, Fx, p + ".fc2.w", p + ".fc2.b", q, D, res=q)
             src_q = q
+        # without a cross layer no attention op has joined the lanes: the fusion tail reads the side lane's text features
+        # and float mask, so its first op joins them
+        tail_join = len(self.ops) if n_layers == 0 and not cached else None
         fused = self._buf("fused", f32, B, D)
         attp = self._buf("attended_pooled", f32, B, D)
         txtp = self._buf("text_pooled", f32, B, D)
@@ -1179,6 +1187,8 @@ class Program(OpList):
         else:
             self._op("pool_gate_ln", "fusion.tail", dict(B=B, L=L, D=D, use_gate=0, phase=0, no_round=self.out_mode),
                      dict(tail_p, cat=fused_h), dict(eps=1e-5))
+        if tail_join is not None:
+            self.ops[tail_join].lane |= LANE_JOIN
 
         # ================= answer head =================
         NA = cfg["num_answers"]
